@@ -2,6 +2,7 @@
 """Benchmark of the hot path: fused HDR merge throughput in Gpix*exposures/s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg2|cfg1]
+                    [--dump-outputs DIR]
 
 One "step" = one fused HDR merge of one synthetic exposure stack (cfg2 of BASELINE.json /
 SURVEY.md 8d by default: 16 exposures 3840x2160x3 uint8 + float64 uncertainty images, dark
@@ -19,6 +20,8 @@ stack -- stacks are independent units, no data-path collective -- so scaling is 
             workload on this box's host cores.
 --impl reference: the oracle port (the reference is pure Python/NumPy and does not run at HEAD,
             see DESIGN.md) on all host cores, row tiles in a process pool.
+--dump-outputs DIR: after the timed steps, what the last step computed as .npy files (`dump_outputs`).  The
+            synthetic inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -295,6 +298,30 @@ def hbm_peak():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+DUMP_SAMPLES = 1 << 20          # samples of the merged image kept by --dump-outputs: 8 MB per float64 array
+DUMP_SEED = 0
+
+
+def dump_outputs(directory, val, std, flat_means):
+    """`--dump-outputs DIR`: the merged radiance and uncertainty of the last timed step, sampled at the same
+    DUMP_SAMPLES flat indices of the (H, W, C) image (drawn once from a seeded generator, sorted), as
+    DIR/hdr_val.npy and DIR/hdr_std.npy; the indices as DIR/hdr_sample_index.npy; the flat ROI means the step
+    passed to the merge as DIR/flat_roi_means.npy.  All float64 (the indices are exact below 2**53)."""
+    import torch
+    directory = Path(directory)
+    directory.mkdir(parents=True, exist_ok=True)
+    n = val.numel()
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, min(n, DUMP_SAMPLES), replace=False))
+    idx_dev = torch.from_numpy(idx).to(val.device)
+    arrays = {"hdr_val": val.reshape(-1)[idx_dev], "hdr_std": std.reshape(-1)[idx_dev],
+              "hdr_sample_index": idx, "flat_roi_means": flat_means}
+    for name, a in arrays.items():
+        if a is None:
+            continue
+        a = a.cpu().numpy() if isinstance(a, torch.Tensor) else a
+        np.save(directory / f"{name}.npy", a.astype(np.float64))
+
+
 # ----------------------------------------------------------------------------- ours
 def run_ours(args, wl):
     import torch
@@ -326,6 +353,7 @@ def run_ours(args, wl):
     out = (torch.empty((wl["H"], wl["W"], wl["C"]), dtype=torch.float64, device=dev),
            torch.empty((wl["H"], wl["W"], wl["C"]), dtype=torch.float64, device=dev))
     roi = cl.measurand._flat_roi()
+    last = {}                                      # the flat ROI means of the latest step, for --dump-outputs
 
     def step():
         ev0 = torch.cuda.Event(enable_timing=True)
@@ -337,6 +365,7 @@ def run_ours(args, wl):
         ops.hdr_merge(data["dn"], data["std"], t, icrf, diff, darks=data["darks"], dark_threshold=DARK_THRESHOLD,
                       median_kernel=KERNEL, flat=data["flat"], flat_std=data["flat_std"], flat_means=means,
                       algo=args.algo, out=out)
+        last["flat_roi_means"] = means
         ev1.record()
         return ev0, ev1
 
@@ -362,6 +391,8 @@ def run_ours(args, wl):
     total_ms = float(tmax.item())
     pix_exp = wl["H"] * wl["W"] * wl["N"]
     value = world * pix_exp * args.steps / (total_ms * 1e-3) / 1e9
+    if args.dump_outputs is not None and rank == 0:     # before the STD-table loop below overwrites `out`
+        dump_outputs(args.dump_outputs, out[0], out[1], last["flat_roi_means"])
 
     # ---- the same stack WITHOUT uncertainty images (sigma from the camera's STD table), device resident ----
     std_lut_np = std_table(wl["C"])
@@ -647,7 +678,7 @@ def run_cfg5(args):
     torch.cuda.set_device(dev)
     if CFG5["stacks"] % world:
         raise SystemExit("cfg5 needs a GPU count that divides 64")
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     launches0 = _lib.launch_count()
     sampler = ClockSampler(dev)
     if rank == 0:
@@ -978,7 +1009,14 @@ def main():
                     help="0 auto, 1 generic kernel, 2 staged two-pass kernel, 4 single-pass kernel")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float64; "
+                         "a fixed, seeded sample of the merged image; cfg1 / cfg2 device arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or args.workload == "cfg5"):
+        ap.error("--dump-outputs is supported for the cfg1 / cfg2 device arm only")
     if args.workload == "cfg5" and args.impl == "ours":
         return run_cfg5(args)
     wl = WORKLOADS[args.workload if args.workload in WORKLOADS else "cfg2"]

@@ -92,10 +92,16 @@ def test_k4_kernels_on_two_rank_shards_allreduce_and_finalize():
     procs = [ctx.Process(target=_worker, args=(r, 2, port, n_dev, q)) for r in range(2)]
     for p in procs:
         p.start()
-    out = [q.get(timeout=500) for _ in procs]
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    try:
+        out = [q.get(timeout=500) for _ in procs]
+        for p in procs:
+            p.join(timeout=60)
+            assert p.exitcode == 0
+    finally:                     # a rank left waiting for a failed peer would outlive the test
+        for p in procs:
+            if p.is_alive():
+                p.kill()
+                p.join()
     out.sort(key=lambda x: x[0])
     mean, pca, t, dn, std, params = _problem()
     for use_std in (False, True):

@@ -39,8 +39,10 @@ def pair_sums(curve, lo, hi, dn, std, t):
 
 def _worker(rank, world, port, q):
     sys.path.insert(0, str(ROOT))
+    # init_from_env selects the rank's GPU when CUDA is present: with fewer GPUs than ranks they share them
+    n_dev = torch.cuda.device_count()
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
-                      LOCAL_RANK=str(rank))
+                      LOCAL_RANK=str(rank % n_dev if n_dev else rank))
     from camera_linearity_b200 import parallel
     from oracle import icrf_energy as oe
     r, w, _ = parallel.init_from_env(backend="gloo")
@@ -95,10 +97,16 @@ def test_pair_sum_allreduce_world_size_2():
     procs = [ctx.Process(target=_worker, args=(r, 2, port, q)) for r in range(2)]
     for p in procs:
         p.start()
-    out = [q.get(timeout=240) for _ in procs]
-    for p in procs:
-        p.join(timeout=60)
-        assert p.exitcode == 0
+    try:
+        out = [q.get(timeout=240) for _ in procs]
+        for p in procs:
+            p.join(timeout=60)
+            assert p.exitcode == 0
+    finally:                     # a rank left waiting for a failed peer would outlive the test
+        for p in procs:
+            if p.is_alive():
+                p.kill()
+                p.join()
     out.sort()
     assert out[0][1] == 0 and out[0][2] == out[1][1] and out[1][2] == 31 * 17      # shards tile the pixels
     for _, _, _, results in out:
