@@ -96,10 +96,14 @@ SIGNATURES = {
     "cl_icrf_energy_workspace_bytes": (_sz, [C.POINTER(IcrfProblem), _i64]),
     "cl_icrf_energy_partial": (_i, [C.POINTER(IcrfProblem), _vp, _vp, _vp, C.POINTER(C.c_double),
                                     _i64, _vp, _vp, _sz, _vp]),
+    "cl_icrf_energy_partial_u16": (_i, [C.POINTER(IcrfProblem), _vp, _vp, _vp, C.POINTER(C.c_double),
+                                        _i64, _vp, _vp, _sz, _vp]),
     "cl_icrf_energy_finalize": (_i, [C.POINTER(IcrfProblem), _vp, _vp, _vp, _vp]),
     "cl_icrf_exchange_bytes": (_sz, [C.POINTER(IcrfProblem), _i]),
     "cl_icrf_energy_population": (_i, [C.POINTER(IcrfProblem), _vp, _vp, _vp, C.POINTER(C.c_double), _i64, _vp, _vp,
                                        _vp, _vp, _sz, C.POINTER(PeerGroup), C.POINTER(DeSelectArgs), _vp]),
+    "cl_icrf_energy_population_u16": (_i, [C.POINTER(IcrfProblem), _vp, _vp, _vp, C.POINTER(C.c_double), _i64, _vp,
+                                           _vp, _vp, _vp, _sz, C.POINTER(PeerGroup), C.POINTER(DeSelectArgs), _vp]),
     "cl_peer_alloc": (_i, [_sz, C.POINTER(C.c_void_p), C.POINTER(IpcHandle)]),
     "cl_peer_open": (_i, [C.POINTER(IpcHandle), C.POINTER(C.c_void_p)]),
     "cl_peer_close": (_i, [_vp]),

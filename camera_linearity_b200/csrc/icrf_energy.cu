@@ -30,7 +30,13 @@
 // flag on each peer, waits for the peers' flags and sums the W contributions in rank order -- so every rank
 // finalises identical numbers without an NCCL launch (one fused kernel instead of reduce + all-reduce +
 // finalize).  Bound: FP64 pipe + shared-memory gathers; the 2-18 MB of pixel data stay in L2.
+//
+// 16-bit cameras (uint16 samples, curves of up to 65536 points): the curves are built by one thread-block cluster per
+// candidate and the partial kernel gathers its table rows from global memory (L1 / L2) instead of shared memory --
+// see curves_wide_kernel and GLOBAL_TABLES below.
 #include "de_common.cuh"
+
+#include <cooperative_groups.h>
 
 #include <cstring>
 
@@ -144,6 +150,134 @@ __global__ void de_trial_curves_kernel(const cl_icrf_problem prob, const double*
     build_curve(prob, mean_icrf, pca, sp, s, curves, valid, tables, sc);
 }
 
+// ---- candidate curves for 256 < D <= 65536 (16-bit cameras: D = 65536; 12-bit data in uint16: D = 4096) ----------
+// One thread-block cluster per candidate: CTA r of the cluster owns the points [r * chunk, (r + 1) * chunk).  Every
+// CTA recomputes the few points it needs from elsewhere -- curve[D-1] (the shift), curve[lower], curve[upper] and the
+// left neighbour of its first point -- with build_curve's arithmetic, so it gets the same bits.  The gates of the
+// eight CTAs meet through distributed shared memory and a cluster barrier; only then are the table rows written
+// (a gated candidate gets the benign table).  One launch, no scratch to clear: capturable in a CUDA graph.
+constexpr int kWideCluster = 8, kWideThreads = 1024;
+constexpr int kMaxSharedDatapoints = 256;      // tables staged in shared memory up to this curve length
+constexpr int kMaxDatapoints = 65536;
+
+__host__ __device__ inline int wide_chunk(int D) { return (D + kWideCluster - 1) / kWideCluster; }
+inline size_t wide_curve_smem(int D) { return (size_t)(wide_chunk(D) + 1) * sizeof(double); }
+
+// curve[d] before the shift (:34-44): matmul(PCA_array, params) summed in order, plus the mean ICRF or linspace ** p[0].
+// The same operations as build_curve, which keeps its own copy so that the D <= 256 kernels compile as before.
+__device__ __forceinline__ double raw_point(const cl_icrf_problem& prob, const double* __restrict__ mean_icrf,
+                                            const double* __restrict__ pca, const double* p, int d) {
+    const int D = prob.datapoints;
+    const int n_pc = prob.use_mean_icrf ? prob.n_params : prob.n_params - 1;
+    const double* coef = prob.use_mean_icrf ? p : p + 1;
+    double acc = 0.0;                       // matmul(PCA_array, params), :38-40
+    for (int k = 0; k < n_pc; ++k) acc = __dadd_rn(acc, __dmul_rn(pca[d * n_pc + k], coef[k]));
+    double base;
+    if (prob.use_mean_icrf) {
+        base = mean_icrf[d];
+    } else {                                // linspace(0, 1, BITS) ** p[0], :37
+        const double x = (d == D - 1) ? 1.0 : __dmul_rn((double)d, __ddiv_rn(1.0, (double)(D - 1)));
+        base = pow(x, p[0]);
+    }
+    return __dadd_rn(base, acc);
+}
+
+// Curve point d of candidate s (value v, its gate decision `bad`, the curve's values lo / hi at the data limits) into
+// `curves` and the I / R tables.
+__device__ __forceinline__ void store_point(const cl_icrf_problem& prob, int s, int d, double v, int bad, double lo,
+                                            double hi, double* __restrict__ curves, double* __restrict__ tables) {
+    const int D = prob.datapoints;
+    curves[(int64_t)s * D + d] = v;
+    const bool masked = v < lo || v > hi;                                                   // :97-98
+    const int64_t at = ((int64_t)(s / kGroup) * D + d) * kGroup + (s % kGroup);
+    if (uniform_masks(prob)) {          // masked entries contribute |0 * x - 1| = 1, subtracted by the kernel
+        // A gated candidate's energy is +inf whatever its sums are, and its curve need not be monotone, so its
+        // own mask could zero entries INSIDE the DN range; the weighted pixel loop would take those for
+        // zero-variance pairs and walk its pixels a second time.  It gets the benign table 1 on [lower, upper].
+        const bool inside = d >= prob.lower && d <= prob.upper;
+        tables[at] = bad ? (inside ? 1.0 : 0.0) : (masked ? 0.0 : v);
+        tables[(int64_t)prob.n_candidates * D + at] = bad ? (inside ? 1.0 : 0.0) : (masked ? 0.0 : 1.0 / v);
+    } else {
+        const double m = masked ? __longlong_as_double(0x7ff8000000000000LL) : v;
+        tables[at] = m;
+        tables[(int64_t)prob.n_candidates * D + at] = 1.0 / m;
+    }
+}
+
+__device__ __forceinline__ void build_curve_wide(const cl_icrf_problem& prob, const double* __restrict__ mean_icrf,
+                                                 const double* __restrict__ pca, const double* p, int s,
+                                                 double* __restrict__ curves, int32_t* __restrict__ valid,
+                                                 double* __restrict__ tables,
+                                                 double* sc /* shared [chunk + 1] */, int* gate /* shared */) {
+    namespace cg = cooperative_groups;
+    cg::cluster_group cluster = cg::this_cluster();
+    const int D = prob.datapoints, rank = (int)cluster.block_rank();
+    const int first = rank * wide_chunk(D), end = min(D, first + wide_chunk(D));
+    const double shift = __dsub_rn(1.0, raw_point(prob, mean_icrf, pca, p, D - 1));    // ICRF += 1 - ICRF[-1], :167
+    auto point = [&](int d) {                                                           // ICRF[0] = 0, :168
+        return d == 0 ? 0.0 : __dadd_rn(raw_point(prob, mean_icrf, pca, p, d), shift);
+    };
+    double* v = sc + 1;                          // v[i] = curve[first + i], sc[0] = curve[first - 1]
+    for (int i = threadIdx.x; first + i < end; i += blockDim.x) v[i] = point(first + i);
+    if (threadIdx.x == 0 && first > 0) sc[0] = point(first - 1);
+    __syncthreads();
+    int bad = 0;
+    for (int i = threadIdx.x; first + i < end; i += blockDim.x) {
+        const double x = v[i];
+        if (x > 1.0 || x < 0.0) bad = 1;                        // :174
+        if (first + i > 0 && !(x > v[i - 1])) bad = 1;          // :178, across the CTA boundary through sc[0]
+        if (x != x) bad = 1;
+    }
+    bad = __syncthreads_or(bad);
+    if (threadIdx.x == 0) *gate = bad;
+    cluster.sync();                              // every CTA's gate is in its shared memory
+    int any = 0;
+    if ((int)threadIdx.x < kWideCluster) any = *cluster.map_shared_rank(gate, (unsigned)threadIdx.x);
+    any = __syncthreads_or(any);
+    cluster.sync();                              // the peers' gates are read before any CTA of the cluster exits
+    const double lo = point(prob.lower), hi = point(prob.upper);                        // :182-183
+    for (int i = threadIdx.x; first + i < end; i += blockDim.x)
+        store_point(prob, s, first + i, v[i], any, lo, hi, curves, tables);
+    if (rank == 0 && threadIdx.x == 0) valid[s] = any ? 0 : 1;
+}
+
+__global__ void __cluster_dims__(kWideCluster, 1, 1) __launch_bounds__(kWideThreads, 1)
+curves_wide_kernel(const cl_icrf_problem prob, const double* __restrict__ mean_icrf, const double* __restrict__ pca,
+                   const double* __restrict__ params, double* __restrict__ curves, int32_t* __restrict__ valid,
+                   double* __restrict__ tables) {
+    extern __shared__ double sc_wide[];
+    __shared__ int gate;
+    const int s = blockIdx.x / kWideCluster;
+    build_curve_wide(prob, mean_icrf, pca, params + (int64_t)s * prob.n_params, s, curves, valid, tables, sc_wide, &gate);
+}
+
+// de_trial_curves_kernel for D > 256: the draws are counter based, so every CTA of the cluster re-derives its
+// member's trial vector; CTA 0 of the cluster writes `trial` / `params`.
+__global__ void __cluster_dims__(kWideCluster, 1, 1) __launch_bounds__(kWideThreads, 1)
+de_trial_curves_wide_kernel(const cl_icrf_problem prob, const double* __restrict__ pop, int n_members,
+                            const de::TrialConfig cfg, const int64_t* __restrict__ generation,
+                            const double* __restrict__ lo, const double* __restrict__ hi, double* __restrict__ trial,
+                            double* __restrict__ params, const double* __restrict__ mean_icrf,
+                            const double* __restrict__ pca, double* __restrict__ curves, int32_t* __restrict__ valid,
+                            double* __restrict__ tables) {
+    extern __shared__ double sc_wide[];
+    __shared__ double sp[64];
+    __shared__ int gate;
+    const int s = blockIdx.x / kWideCluster, P = prob.n_params;
+    const bool writer = blockIdx.x % kWideCluster == 0;
+    if ((int)threadIdx.x < P) {
+        double tv = 0.0, pv = 0.0;
+        if (s < n_members) {
+            de::trial_component(pop, n_members, P, cfg, (uint64_t)generation[0], s, threadIdx.x, lo, hi, tv, pv);
+            if (writer) trial[s * P + threadIdx.x] = tv;
+        }
+        if (writer) params[s * P + threadIdx.x] = pv;  // padding members (s >= n_members) evaluate the zero vector
+        sp[threadIdx.x] = pv;
+    }
+    __syncthreads();
+    build_curve_wide(prob, mean_icrf, pca, sp, s, curves, valid, tables, sc_wide, &gate);
+}
+
 // ---- partial energies -----------------------------------------------------------------------------
 // One pixel per warp-iteration, two pixels in flight (the DN / sigma loads of the next pixel are
 // issued before the arithmetic of the current one).
@@ -153,8 +287,8 @@ struct PixelData {
     double sg[USE_STD ? N : 1];
 };
 
-template <int N, bool USE_STD>
-__device__ __forceinline__ void load_pixel(PixelData<N, USE_STD>& d, const uint8_t* __restrict__ dn,
+template <int N, bool USE_STD, typename DN>
+__device__ __forceinline__ void load_pixel(PixelData<N, USE_STD>& d, const DN* __restrict__ dn,
                                            const double* __restrict__ sd, int64_t px, int D) {
 #pragma unroll
     for (int k = 0; k < N; ++k) {
@@ -335,22 +469,34 @@ __device__ __forceinline__ void accumulate_pixel(const PixelData<N, USE_STD>& d,
     }
 }
 
-template <int N, bool USE_STD, int WARPS, bool UNIFORM>
+// DN: uint8_t or uint16_t samples.  GLOBAL_TABLES (D > 256): the candidate group's [dn][lane] tables stay in global
+// memory -- 2 x D x 32 x 8 B is 32 MB at D = 65536 -- and every gather is still one contiguous 256-byte row per warp,
+// served by L1 / L2 (the whole blob, 2 x S x D x 8 B = 64 MiB at S = 64, fits the 126 MB L2 next to the pixels).
+template <int N, bool USE_STD, int WARPS, bool UNIFORM, typename DN = uint8_t, bool GLOBAL_TABLES = false>
 __global__ void __launch_bounds__(WARPS * 32, 1)
-energy_partial_kernel(const double* __restrict__ tables, int D, int S, const uint8_t* __restrict__ dn,
+energy_partial_kernel(const double* __restrict__ tables, int D, int S, const DN* __restrict__ dn,
                       const double* __restrict__ sd, int64_t n_pixels, int64_t px_per_cta,
                       const __grid_constant__ ExposureScales sc, int lower, int upper,
                       double* __restrict__ cta_partial /* [cta][S][pairs][2] */) {
     constexpr int P = N * (N - 1) / 2;
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    double* tabI = reinterpret_cast<double*>(smem_raw);            // [D][32]
-    double* tabR = tabI + D * kGroup;                              // [D][32]
     const int group = blockIdx.y;
     const double* srcI = tables + (int64_t)group * D * kGroup;
     const double* srcR = srcI + (int64_t)S * D;
-    for (int i = threadIdx.x; i < D * kGroup; i += WARPS * 32) {
-        tabI[i] = srcI[i];
-        tabR[i] = srcR[i];
+    const double* tabI;
+    const double* tabR;
+    if constexpr (GLOBAL_TABLES) {
+        tabI = srcI;                                               // [D][32], D * 32 < 2^31
+        tabR = srcR;
+    } else {
+        double* stI = reinterpret_cast<double*>(smem_raw);         // [D][32]
+        double* stR = stI + D * kGroup;                            // [D][32]
+        for (int i = threadIdx.x; i < D * kGroup; i += WARPS * 32) {
+            stI[i] = srcI[i];
+            stR[i] = srcR[i];
+        }
+        tabI = stI;
+        tabR = stR;
     }
     const int64_t first = (int64_t)blockIdx.x * px_per_cta;
     const int64_t last = min(n_pixels, first + px_per_cta);
@@ -646,10 +792,19 @@ struct Plan {
     int64_t px_per_cta;
 };
 
+// CTAs per SM of the partial kernel when its tables stay in global memory (D > 256): nothing to stage, so several
+// CTAs share an SM and hide the L2 latency of the gathers (see DESIGN.md, K4 for D > 256).
+#ifndef CL_K4_GLOBAL_CTAS_PER_SM
+#define CL_K4_GLOBAL_CTAS_PER_SM 2
+#endif
+constexpr int kGlobalCtasPerSm = CL_K4_GLOBAL_CTAS_PER_SM;
+
+inline bool global_tables(const cl_icrf_problem& p) { return p.datapoints > kMaxSharedDatapoints; }
+
 inline Plan make_plan(const cl_icrf_problem& p, int64_t n_pixels) {
     Plan pl;
     pl.groups = p.n_candidates / kGroup;
-    int chunks = sm_count() / (pl.groups > 0 ? pl.groups : 1);
+    int chunks = (global_tables(p) ? kGlobalCtasPerSm : 1) * sm_count() / (pl.groups > 0 ? pl.groups : 1);
     if (chunks < 1) chunks = 1;
     const int64_t min_px = 16 * 8;         // do not split tiny problems into idle CTAs
     if ((int64_t)chunks * min_px > n_pixels) chunks = (int)((n_pixels + min_px - 1) / min_px);
@@ -659,18 +814,45 @@ inline Plan make_plan(const cl_icrf_problem& p, int64_t n_pixels) {
     return pl;
 }
 
-inline bool problem_ok(const cl_icrf_problem* p) {
+// max_datapoints: 256 for the uint8 entry points, 65536 for the others
+inline bool problem_ok(const cl_icrf_problem* p, int max_datapoints = kMaxDatapoints) {
     return p && p->n_candidates >= kGroup && p->n_candidates % kGroup == 0 && p->n_params >= 1 &&
-           p->n_params <= 64 && p->datapoints >= 2 && p->datapoints <= 256 && p->lower >= 0 &&
+           p->n_params <= 64 && p->datapoints >= 2 && p->datapoints <= max_datapoints && p->lower >= 0 &&
            p->lower < p->datapoints && p->upper >= 0 && p->upper < p->datapoints && p->n_exposures >= 2 &&
            p->n_exposures <= kMaxN && (p->use_mean_icrf || p->n_params >= 2);
 }
 
-template <int N>
-int launch_partial(const cl_icrf_problem& p, const Plan& pl, const double* tables, const uint8_t* dn,
+// D > 256: tables read from global memory, shared memory only for the warp reduction
+template <int N, typename DN>
+int launch_partial_global(const cl_icrf_problem& p, const Plan& pl, const double* tables, const DN* dn,
+                          const double* sd, int64_t n_pixels, const ExposureScales& sc, double* cta_partial,
+                          cudaStream_t stream) {
+    // registers: 2P accumulators per lane; no spills at N = 6 with std needs more than 128 (a register cap for two
+    // resident CTAs spills the accumulators at every N >= 4)
+    constexpr int WARPS = N <= 5 ? 16 : 8;
+    const size_t smem = (size_t)(WARPS / 2) * 2 * n_pairs(N) * 32 * sizeof(double);
+    dim3 grid(pl.chunks, pl.groups);
+    auto go = [&](auto kernel) -> int {
+        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return cuda_status(e);
+        kernel<<<grid, WARPS * 32, smem, stream>>>(tables, p.datapoints, p.n_candidates, dn, sd, n_pixels,
+                                                   pl.px_per_cta, sc, p.lower, p.upper, cta_partial);
+        return launched();
+    };
+    if (uniform_masks(p))
+        return sd ? go(energy_partial_kernel<N, true, WARPS, true, DN, true>)
+                  : go(energy_partial_kernel<N, false, WARPS, true, DN, true>);
+    return sd ? go(energy_partial_kernel<N, true, WARPS, false, DN, true>)
+              : go(energy_partial_kernel<N, false, WARPS, false, DN, true>);
+}
+
+template <int N, typename DN>
+int launch_partial(const cl_icrf_problem& p, const Plan& pl, const double* tables, const DN* dn,
                    const double* sd, int64_t n_pixels, const ExposureScales& sc, double* cta_partial,
                    cudaStream_t stream) {
     constexpr int WARPS = N <= 6 ? 16 : 8;         // registers: 2P accumulators per lane
+    if constexpr (sizeof(DN) > 1)                 // (the uint8 entry points accept D <= 256 only)
+        if (global_tables(p)) return launch_partial_global<N>(p, pl, tables, dn, sd, n_pixels, sc, cta_partial, stream);
     const size_t tab_bytes = (size_t)p.datapoints * kGroup * 2 * sizeof(double);
     const size_t red_bytes = (size_t)(WARPS / 2) * 2 * n_pairs(N) * 32 * sizeof(double);
     const size_t smem = tab_bytes > red_bytes ? tab_bytes : red_bytes;
@@ -683,11 +865,14 @@ int launch_partial(const cl_icrf_problem& p, const Plan& pl, const double* table
         return launched();
     };
     if (uniform_masks(p))
-        return sd ? go(energy_partial_kernel<N, true, WARPS, true>) : go(energy_partial_kernel<N, false, WARPS, true>);
-    return sd ? go(energy_partial_kernel<N, true, WARPS, false>) : go(energy_partial_kernel<N, false, WARPS, false>);
+        return sd ? go(energy_partial_kernel<N, true, WARPS, true, DN>)
+                  : go(energy_partial_kernel<N, false, WARPS, true, DN>);
+    return sd ? go(energy_partial_kernel<N, true, WARPS, false, DN>)
+              : go(energy_partial_kernel<N, false, WARPS, false, DN>);
 }
 
-int run_partial(const cl_icrf_problem* p, const void* tables, const uint8_t* dn, const double* std,
+template <typename DN>
+int run_partial(const cl_icrf_problem* p, const void* tables, const DN* dn, const double* std,
                 const double* exposure_s, int64_t n_pixels, double* cta_partial, const Plan& pl, cudaStream_t s) {
     const int N = p->n_exposures;
     ExposureScales sc;
@@ -716,54 +901,16 @@ inline size_t partial_bytes(const cl_icrf_problem& p, const Plan& pl) {
 }  // namespace
 }  // namespace cl
 
-extern "C" {
+extern "C" size_t cl_icrf_energy_workspace_bytes(const cl_icrf_problem* p, int64_t n_pixels);
 
-size_t cl_icrf_tables_bytes(const cl_icrf_problem* p) {
-    if (!cl::problem_ok(p)) return 0;
-    return (size_t)p->n_candidates * p->datapoints * 2 * sizeof(double);
-}
+namespace cl {
+namespace {
 
-int cl_icrf_curves(const cl_icrf_problem* p, const double* mean_icrf, const double* pca,
-                   const double* params, double* curves, int32_t* valid, void* tables, void* stream) {
-    using namespace cl;
-    if (!problem_ok(p)) return CL_ERR_INVALID_ARGUMENT;
-    CL_REQUIRE(pca && params && curves && valid && tables);
-    CL_REQUIRE(mean_icrf || !p->use_mean_icrf);
-    if (!aligned(tables, 16)) return CL_ERR_ALIGNMENT;
-    curves_kernel<<<p->n_candidates, 256, 0, (cudaStream_t)stream>>>(
-        *p, mean_icrf, pca, params, curves, valid, reinterpret_cast<double*>(tables));
-    return launched();
-}
-
-int cl_de_trial_curves(const cl_icrf_problem* p, const double* pop, int n_members, double dither_lo, double dither_hi,
-                       double crossover, uint64_t seed, const int64_t* generation, const double* lower,
-                       const double* upper, double* trial, double* params, const double* mean_icrf,
-                       const double* pca, double* curves, int32_t* valid, void* tables, void* stream) {
-    using namespace cl;
-    if (!problem_ok(p)) return CL_ERR_INVALID_ARGUMENT;
-    CL_REQUIRE(pop && generation && lower && upper && trial && params && pca && curves && valid && tables);
-    CL_REQUIRE(mean_icrf || !p->use_mean_icrf);
-    CL_REQUIRE(n_members >= 4 && n_members <= p->n_candidates);
-    CL_REQUIRE(dither_lo <= dither_hi && crossover >= 0.0 && crossover <= 1.0);
-    if (!aligned(tables, 16)) return CL_ERR_ALIGNMENT;
-    const de::TrialConfig cfg{dither_lo, dither_hi, crossover, seed};
-    de_trial_curves_kernel<<<p->n_candidates, 256, 0, (cudaStream_t)stream>>>(
-        *p, pop, n_members, cfg, generation, lower, upper, trial, params, mean_icrf, pca, curves, valid,
-        reinterpret_cast<double*>(tables));
-    return launched();
-}
-
-size_t cl_icrf_energy_workspace_bytes(const cl_icrf_problem* p, int64_t n_pixels) {
-    if (!cl::problem_ok(p) || n_pixels < 0) return 0;
-    const cl::Plan pl = cl::make_plan(*p, n_pixels > 0 ? n_pixels : 1);
-    return cl::partial_bytes(*p, pl) + 16;
-}
-
-int cl_icrf_energy_partial(const cl_icrf_problem* p, const void* tables, const uint8_t* dn,
-                           const double* std, const double* exposure_s, int64_t n_pixels,
-                           double* pair_acc, void* workspace, size_t workspace_bytes, void* stream) {
-    using namespace cl;
-    if (!problem_ok(p)) return CL_ERR_INVALID_ARGUMENT;
+template <typename DN>
+int energy_partial(const cl_icrf_problem* p, int max_datapoints, const void* tables, const DN* dn, const double* std,
+                   const double* exposure_s, int64_t n_pixels, double* pair_acc, void* workspace,
+                   size_t workspace_bytes, void* stream) {
+    if (!problem_ok(p, max_datapoints)) return CL_ERR_INVALID_ARGUMENT;
     CL_REQUIRE(tables && exposure_s && pair_acc && n_pixels >= 0);
     CL_REQUIRE(n_pixels == 0 || dn);
     CL_REQUIRE((p->use_std != 0) == (std != nullptr) || n_pixels == 0);
@@ -781,28 +928,12 @@ int cl_icrf_energy_partial(const cl_icrf_problem* p, const void* tables, const u
     return launched();
 }
 
-int cl_icrf_energy_finalize(const cl_icrf_problem* p, const double* pair_acc, const int32_t* valid,
-                            double* energy, void* stream) {
-    using namespace cl;
-    if (!problem_ok(p)) return CL_ERR_INVALID_ARGUMENT;
-    CL_REQUIRE(pair_acc && valid && energy);
-    finalize_kernel<<<(p->n_candidates + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        pair_acc, valid, p->n_candidates, n_pairs(p->n_exposures), energy);
-    return launched();
-}
-
-size_t cl_icrf_exchange_bytes(const cl_icrf_problem* p, int world) {
-    if (!cl::problem_ok(p) || world < 1 || world > CL_MAX_PEERS) return 0;
-    const size_t per_rank = (size_t)p->n_candidates * cl::n_pairs(p->n_exposures) * 2 * sizeof(double);
-    return 2 * (size_t)world * per_rank + (size_t)CL_MAX_PEERS * sizeof(uint64_t) + 64;   // slots, flags, seq + ticket
-}
-
-int cl_icrf_energy_population(const cl_icrf_problem* p, const void* tables, const uint8_t* dn, const double* std,
-                              const double* exposure_s, int64_t n_pixels, const int32_t* valid, double* pair_acc,
-                              double* energy, void* workspace, size_t workspace_bytes, const cl_peer_group* peers,
-                              const cl_de_select_args* select, void* stream) {
-    using namespace cl;
-    if (!problem_ok(p)) return CL_ERR_INVALID_ARGUMENT;
+template <typename DN>
+int energy_population(const cl_icrf_problem* p, int max_datapoints, const void* tables, const DN* dn,
+                      const double* std, const double* exposure_s, int64_t n_pixels, const int32_t* valid,
+                      double* pair_acc, double* energy, void* workspace, size_t workspace_bytes,
+                      const cl_peer_group* peers, const cl_de_select_args* select, void* stream) {
+    if (!problem_ok(p, max_datapoints)) return CL_ERR_INVALID_ARGUMENT;
     CL_REQUIRE(tables && exposure_s && valid && pair_acc && energy && n_pixels >= 1 && dn && peers);
     CL_REQUIRE((p->use_std != 0) == (std != nullptr));
     CL_REQUIRE(peers->world >= 1 && peers->world <= CL_MAX_PEERS && peers->rank >= 0 && peers->rank < peers->world);
@@ -840,6 +971,116 @@ int cl_icrf_energy_population(const cl_icrf_problem* p, const void* tables, cons
                                                        pg, reinterpret_cast<uint64_t*>(tail),
                                                        reinterpret_cast<unsigned int*>(tail + 8), sel);
     return launched();
+}
+
+}  // namespace
+}  // namespace cl
+
+extern "C" {
+
+size_t cl_icrf_tables_bytes(const cl_icrf_problem* p) {
+    if (!cl::problem_ok(p)) return 0;
+    return (size_t)p->n_candidates * p->datapoints * 2 * sizeof(double);
+}
+
+int cl_icrf_curves(const cl_icrf_problem* p, const double* mean_icrf, const double* pca,
+                   const double* params, double* curves, int32_t* valid, void* tables, void* stream) {
+    using namespace cl;
+    if (!problem_ok(p)) return CL_ERR_INVALID_ARGUMENT;
+    CL_REQUIRE(pca && params && curves && valid && tables);
+    CL_REQUIRE(mean_icrf || !p->use_mean_icrf);
+    if (!aligned(tables, 16)) return CL_ERR_ALIGNMENT;
+    if (p->datapoints > kMaxSharedDatapoints) {
+        const size_t smem = wide_curve_smem(p->datapoints);
+        cudaError_t e = cudaFuncSetAttribute(curves_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return cuda_status(e);
+        curves_wide_kernel<<<p->n_candidates * kWideCluster, kWideThreads, smem, (cudaStream_t)stream>>>(
+            *p, mean_icrf, pca, params, curves, valid, reinterpret_cast<double*>(tables));
+        return launched();
+    }
+    curves_kernel<<<p->n_candidates, 256, 0, (cudaStream_t)stream>>>(
+        *p, mean_icrf, pca, params, curves, valid, reinterpret_cast<double*>(tables));
+    return launched();
+}
+
+int cl_de_trial_curves(const cl_icrf_problem* p, const double* pop, int n_members, double dither_lo, double dither_hi,
+                       double crossover, uint64_t seed, const int64_t* generation, const double* lower,
+                       const double* upper, double* trial, double* params, const double* mean_icrf,
+                       const double* pca, double* curves, int32_t* valid, void* tables, void* stream) {
+    using namespace cl;
+    if (!problem_ok(p)) return CL_ERR_INVALID_ARGUMENT;
+    CL_REQUIRE(pop && generation && lower && upper && trial && params && pca && curves && valid && tables);
+    CL_REQUIRE(mean_icrf || !p->use_mean_icrf);
+    CL_REQUIRE(n_members >= 4 && n_members <= p->n_candidates);
+    CL_REQUIRE(dither_lo <= dither_hi && crossover >= 0.0 && crossover <= 1.0);
+    if (!aligned(tables, 16)) return CL_ERR_ALIGNMENT;
+    const de::TrialConfig cfg{dither_lo, dither_hi, crossover, seed};
+    if (p->datapoints > kMaxSharedDatapoints) {
+        const size_t smem = wide_curve_smem(p->datapoints);
+        cudaError_t e =
+            cudaFuncSetAttribute(de_trial_curves_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        if (e != cudaSuccess) return cuda_status(e);
+        de_trial_curves_wide_kernel<<<p->n_candidates * kWideCluster, kWideThreads, smem, (cudaStream_t)stream>>>(
+            *p, pop, n_members, cfg, generation, lower, upper, trial, params, mean_icrf, pca, curves, valid,
+            reinterpret_cast<double*>(tables));
+        return launched();
+    }
+    de_trial_curves_kernel<<<p->n_candidates, 256, 0, (cudaStream_t)stream>>>(
+        *p, pop, n_members, cfg, generation, lower, upper, trial, params, mean_icrf, pca, curves, valid,
+        reinterpret_cast<double*>(tables));
+    return launched();
+}
+
+size_t cl_icrf_energy_workspace_bytes(const cl_icrf_problem* p, int64_t n_pixels) {
+    if (!cl::problem_ok(p) || n_pixels < 0) return 0;
+    const cl::Plan pl = cl::make_plan(*p, n_pixels > 0 ? n_pixels : 1);
+    return cl::partial_bytes(*p, pl) + 16;
+}
+
+int cl_icrf_energy_partial(const cl_icrf_problem* p, const void* tables, const uint8_t* dn,
+                           const double* std, const double* exposure_s, int64_t n_pixels,
+                           double* pair_acc, void* workspace, size_t workspace_bytes, void* stream) {
+    return cl::energy_partial(p, cl::kMaxSharedDatapoints, tables, dn, std, exposure_s, n_pixels, pair_acc, workspace,
+                              workspace_bytes, stream);
+}
+
+int cl_icrf_energy_partial_u16(const cl_icrf_problem* p, const void* tables, const uint16_t* dn,
+                               const double* std, const double* exposure_s, int64_t n_pixels,
+                               double* pair_acc, void* workspace, size_t workspace_bytes, void* stream) {
+    return cl::energy_partial(p, cl::kMaxDatapoints, tables, dn, std, exposure_s, n_pixels, pair_acc, workspace,
+                              workspace_bytes, stream);
+}
+
+int cl_icrf_energy_finalize(const cl_icrf_problem* p, const double* pair_acc, const int32_t* valid,
+                            double* energy, void* stream) {
+    using namespace cl;
+    if (!problem_ok(p)) return CL_ERR_INVALID_ARGUMENT;
+    CL_REQUIRE(pair_acc && valid && energy);
+    finalize_kernel<<<(p->n_candidates + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
+        pair_acc, valid, p->n_candidates, n_pairs(p->n_exposures), energy);
+    return launched();
+}
+
+size_t cl_icrf_exchange_bytes(const cl_icrf_problem* p, int world) {
+    if (!cl::problem_ok(p) || world < 1 || world > CL_MAX_PEERS) return 0;
+    const size_t per_rank = (size_t)p->n_candidates * cl::n_pairs(p->n_exposures) * 2 * sizeof(double);
+    return 2 * (size_t)world * per_rank + (size_t)CL_MAX_PEERS * sizeof(uint64_t) + 64;   // slots, flags, seq + ticket
+}
+
+int cl_icrf_energy_population(const cl_icrf_problem* p, const void* tables, const uint8_t* dn, const double* std,
+                              const double* exposure_s, int64_t n_pixels, const int32_t* valid, double* pair_acc,
+                              double* energy, void* workspace, size_t workspace_bytes, const cl_peer_group* peers,
+                              const cl_de_select_args* select, void* stream) {
+    return cl::energy_population(p, cl::kMaxSharedDatapoints, tables, dn, std, exposure_s, n_pixels, valid, pair_acc,
+                                 energy, workspace, workspace_bytes, peers, select, stream);
+}
+
+int cl_icrf_energy_population_u16(const cl_icrf_problem* p, const void* tables, const uint16_t* dn, const double* std,
+                                  const double* exposure_s, int64_t n_pixels, const int32_t* valid, double* pair_acc,
+                                  double* energy, void* workspace, size_t workspace_bytes, const cl_peer_group* peers,
+                                  const cl_de_select_args* select, void* stream) {
+    return cl::energy_population(p, cl::kMaxDatapoints, tables, dn, std, exposure_s, n_pixels, valid, pair_acc,
+                                 energy, workspace, workspace_bytes, peers, select, stream);
 }
 
 // ---- peer-visible device buffers (CUDA IPC) for the exchange above ------------------------------------

@@ -427,19 +427,27 @@ def _plan_device(fn):
     return wrapper
 
 
+def _max_dn(dn: Tensor) -> int:
+    """Largest sample of a uint8 / uint16 tensor (torch has no max for uint16: widened to int32 first, never viewed
+    as int16, which would turn 32768..65535 negative)."""
+    return int(dn.max()) if dn.dtype == torch.uint8 else int(dn.to(torch.int32).max())
+
+
 class IcrfEnergyPlan:
     """Device-resident state of one calibration problem (one colour channel): pixel samples,
     PCA basis, scratch.  ``partial()`` and ``finalize()`` map onto the C ABI calls so that a
-    multi-GPU driver can all-reduce the pair sums in between (parallel.py)."""
+    multi-GPU driver can all-reduce the pair sums in between (parallel.py).  uint8 stacks take curves of up to 256
+    points, uint16 stacks (16- / 12-bit cameras) up to 65536 through the ``_u16`` entry points."""
 
     def __init__(self, dn_stack: Tensor, std_stack: Optional[Tensor], exposures, mean_icrf,
                  pca_basis: Tensor, lower: int, upper: int, use_mean_icrf: bool, n_candidates: int):
         dev = _require_cuda(dn_stack, std_stack, pca_basis)
         self.device = dev
         self.lib = _lib.load()
-        if dn_stack.dtype != torch.uint8:
-            raise TypeError("the calibration value stack must be uint8 "
+        if dn_stack.dtype not in (torch.uint8, torch.uint16):
+            raise TypeError("the calibration value stack must be uint8 or uint16 "
                             "(ICRF_calibration_exposure.py:191 indexes the curve with it)")
+        self.wide = dn_stack.dtype == torch.uint16          # 16-bit (or 12-bit) camera: the _u16 entry points
         if dn_stack.ndim != 3:
             raise ValueError("image_stack must be a 3D CuPy array with shape (X, Y, N).")
         n_exp = int(dn_stack.shape[2])
@@ -459,7 +467,7 @@ class IcrfEnergyPlan:
         self.datapoints = int(self.pca.shape[0])
         self.n_pc = int(self.pca.shape[1])
         self.mean = None if mean_icrf is None else _f64c(torch.as_tensor(mean_icrf, device=dev))
-        if self.n_pixels and int(self.dn.max()) >= self.datapoints:
+        if self.n_pixels and _max_dn(self.dn) >= self.datapoints:
             raise IndexError("digital numbers exceed the curve length")
         self.exposures = (C.c_double * n_exp)(*exposures.tolist())
         self.n_real = int(n_candidates)
@@ -507,9 +515,10 @@ class IcrfEnergyPlan:
 
     @_plan_device
     def partial(self) -> Tensor:
-        check(self.lib.cl_icrf_energy_partial(C.byref(self.prob), _ptr(self.tables), _ptr(self.dn), _ptr(self.std),
-                                              self.exposures, self.n_pixels, _ptr(self.pair_acc), _ptr(self.ws),
-                                              self.ws_bytes, _stream()), "cl_icrf_energy_partial")
+        name = "cl_icrf_energy_partial_u16" if self.wide else "cl_icrf_energy_partial"
+        check(getattr(self.lib, name)(C.byref(self.prob), _ptr(self.tables), _ptr(self.dn), _ptr(self.std),
+                                      self.exposures, self.n_pixels, _ptr(self.pair_acc), _ptr(self.ws),
+                                      self.ws_bytes, _stream()), name)
         return self.pair_acc
 
     @_plan_device
@@ -525,11 +534,11 @@ class IcrfEnergyPlan:
         ``_lib.DeSelectArgs`` -- the DE selection of the generation then runs in the same launch."""
         if self.n_pixels == 0:
             raise ValueError("population() needs at least one pixel on every rank")
-        check(self.lib.cl_icrf_energy_population(C.byref(self.prob), _ptr(self.tables), _ptr(self.dn), _ptr(self.std),
-                                                 self.exposures, self.n_pixels, _ptr(self.valid), _ptr(self.pair_acc),
-                                                 _ptr(self.energy), _ptr(self.ws), self.ws_bytes, C.byref(self.peers),
-                                                 None if select is None else C.byref(select), _stream()),
-              "cl_icrf_energy_population")
+        name = "cl_icrf_energy_population_u16" if self.wide else "cl_icrf_energy_population"
+        check(getattr(self.lib, name)(C.byref(self.prob), _ptr(self.tables), _ptr(self.dn), _ptr(self.std),
+                                      self.exposures, self.n_pixels, _ptr(self.valid), _ptr(self.pair_acc),
+                                      _ptr(self.energy), _ptr(self.ws), self.ws_bytes, C.byref(self.peers),
+                                      None if select is None else C.byref(select), _stream()), name)
         return self.energy[: self.n_real]
 
     def evaluate(self, params) -> Tensor:
@@ -927,11 +936,12 @@ def _op_icrf_energy_partial(tables: Tensor, dn: Tensor, std: Optional[Tensor], e
                             n_candidates: int, n_params: int, datapoints: int, use_mean: bool, lower: int,
                             upper: int) -> Tensor:
     """cl_icrf_energy_partial: per-(candidate, exposure pair) numerator / denominator sums over the given pixels,
-    (S, pairs, 2) float64 -- what ranks all-reduce before icrf_energy_finalize."""
+    (S, pairs, 2) float64 -- what ranks all-reduce before icrf_energy_finalize.  A uint16 ``dn`` (16- / 12-bit
+    cameras, datapoints <= 65536) goes to cl_icrf_energy_partial_u16."""
     _require_cuda(tables, dn, std)
     lib = _lib.load()
-    if dn.dtype != torch.uint8 or dn.ndim != 2:
-        raise TypeError("dn must be a (pixels, N) uint8 tensor")
+    if dn.dtype not in (torch.uint8, torch.uint16) or dn.ndim != 2:
+        raise TypeError("dn must be a (pixels, N) uint8 or uint16 tensor")
     n_px, n_exp = (int(v) for v in dn.shape)
     prob = _icrf_problem(n_candidates, n_params, datapoints, use_mean, lower, upper, n_exp, std is not None)
     sd = None if std is None else _f64c(std)
@@ -939,8 +949,9 @@ def _op_icrf_energy_partial(tables: Tensor, dn: Tensor, std: Optional[Tensor], e
     ws_bytes = lib.cl_icrf_energy_workspace_bytes(C.byref(prob), n_px)
     ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=dn.device)
     t = (C.c_double * n_exp)(*[float(x) for x in exposures])
-    check(lib.cl_icrf_energy_partial(C.byref(prob), _ptr(tables), _ptr(dn.contiguous()), _ptr(sd), t, n_px, _ptr(acc),
-                                     _ptr(ws), ws_bytes, _stream()), "cl_icrf_energy_partial")
+    name = "cl_icrf_energy_partial_u16" if dn.dtype == torch.uint16 else "cl_icrf_energy_partial"
+    check(getattr(lib, name)(C.byref(prob), _ptr(tables), _ptr(dn.contiguous()), _ptr(sd), t, n_px, _ptr(acc),
+                             _ptr(ws), ws_bytes, _stream()), name)
     return acc
 
 

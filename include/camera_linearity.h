@@ -192,14 +192,18 @@ int cl_welford_stack(const uint8_t* frames, int n_frames, int64_t n_samples, int
 typedef struct cl_icrf_problem {
     int32_t n_candidates;   /* S, multiple of 32                                            */
     int32_t n_params;       /* 5 (use_mean_icrf) or 6 (exponent + 5), any >= 1              */
-    int32_t datapoints;     /* D = curve length = LUT rows (<= 256)                         */
+    int32_t datapoints;     /* D = curve length = LUT rows (<= 256 for uint8 samples,        */
+                            /* <= 65536 for uint16 samples: the _u16 entry points)           */
     int32_t use_mean_icrf;  /* 1: mean + pca @ p ; 0: linspace(0,1,D)**p[0] + pca @ p[1:]   */
     int32_t lower, upper;   /* data limits as DN indices (ICRF_calibration_exposure.py:182) */
     int32_t n_exposures;    /* N, 2..CL_MAX_PAIR_EXPOSURES                                  */
     int32_t use_std;
 } cl_icrf_problem;
 
-size_t cl_icrf_tables_bytes(const cl_icrf_problem* p);   /* size of the `tables` scratch     */
+/* cl_icrf_tables_bytes, cl_icrf_curves, cl_icrf_energy_workspace_bytes, cl_icrf_energy_finalize, cl_icrf_exchange_bytes
+ * and cl_de_trial_curves accept 2 <= D <= 65536 (D > 256: one thread-block cluster per candidate builds the curve);
+ * the uint8 partial / population calls accept D <= 256, their _u16 forms D <= 65536. */
+size_t cl_icrf_tables_bytes(const cl_icrf_problem* p);   /* size of the `tables` scratch: 2 * S * D * 8 bytes */
 int cl_icrf_curves(const cl_icrf_problem* p, const double* mean_icrf, const double* pca,
                    const double* params /* device [S][n_params] */, double* curves /* [S][D] */,
                    int32_t* valid /* [S] */, void* tables, void* stream);
@@ -210,6 +214,14 @@ int cl_icrf_energy_partial(const cl_icrf_problem* p, const void* tables,
                            const double* exposure_s /* HOST [N] */, int64_t n_pixels,
                            double* pair_acc /* device [S][pairs][2] */, void* workspace,
                            size_t workspace_bytes, void* stream);
+/* The same for 16-bit (or 12-bit) cameras: dn is device [n_pixels][N] uint16, every dn < D <= 65536.  For D > 256 the
+ * tables are gathered from global memory (L2) instead of being staged in shared memory. */
+int cl_icrf_energy_partial_u16(const cl_icrf_problem* p, const void* tables,
+                               const uint16_t* dn /* device [n_pixels][N] */,
+                               const double* std /* device [n_pixels][N] or NULL */,
+                               const double* exposure_s /* HOST [N] */, int64_t n_pixels,
+                               double* pair_acc /* device [S][pairs][2] */, void* workspace,
+                               size_t workspace_bytes, void* stream);
 int cl_icrf_energy_finalize(const cl_icrf_problem* p, const double* pair_acc,
                             const int32_t* valid, double* energy /* device [S] */, void* stream);
 
@@ -246,6 +258,13 @@ int cl_icrf_energy_population(const cl_icrf_problem* p, const void* tables, cons
                               double* pair_acc, double* energy, void* workspace, size_t workspace_bytes,
                               const cl_peer_group* peers, const cl_de_select_args* select /* nullable */,
                               void* stream);
+/* cl_icrf_energy_population for uint16 samples (dn < D <= 65536); the exchange buffers and the peer route are the
+ * same as for uint8 (cl_icrf_exchange_bytes depends on neither D nor the sample type). */
+int cl_icrf_energy_population_u16(const cl_icrf_problem* p, const void* tables, const uint16_t* dn,
+                                  const double* std, const double* exposure_s /* HOST [N] */, int64_t n_pixels,
+                                  const int32_t* valid, double* pair_acc, double* energy, void* workspace,
+                                  size_t workspace_bytes, const cl_peer_group* peers,
+                                  const cl_de_select_args* select /* nullable */, void* stream);
 
 /* Peer-visible device buffers (CUDA IPC) for the exchange above: cl_peer_alloc on the owning rank (cudaMalloc,
  * zero-filled, synchronous), the 64-byte handle travels to the other processes by any means
@@ -303,7 +322,8 @@ int cl_de_trial(const double* pop, int n_members, int n_params, double dither_lo
                 double crossover, uint64_t seed, const int64_t* generation, const double* lower,
                 const double* upper, double* trial, double* params, void* stream);
 /* cl_de_trial fused with cl_icrf_curves (one launch: CTA s draws member s's trial vector and builds its curve
- * and tables).  n_members <= p->n_candidates; the padding candidates evaluate the zero parameter vector. */
+ * and tables; D > 256: every CTA of candidate s's cluster draws it, one writes trial / params).
+ * n_members <= p->n_candidates; the padding candidates evaluate the zero parameter vector. */
 int cl_de_trial_curves(const cl_icrf_problem* p, const double* pop, int n_members, double dither_lo,
                        double dither_hi, double crossover, uint64_t seed, const int64_t* generation,
                        const double* lower, const double* upper, double* trial, double* params,
