@@ -7,10 +7,10 @@
 // (DN bytes only), pass B re-reads the DNs (L1/L2 hits) together with the float64 std stream and
 // accumulates value and variance in float64 registers.  Weight / ICRF tables are pre-multiplied
 // ({w}, {w*g, dICRF}) and live in shared memory for 8-bit data, in an L2-resident workspace for
-// 16-bit data.  The fast path for 8-bit RGB/mono stacks is hdr_merge_staged.cu ("algo 2"), the one for
-// 16-bit stacks hdr_merge_wide.cu ("algo 3").
+// 16-bit data.  Which kernel runs for a stack: the selection table above cl_hdr_merge.
 #include "hdr_merge.cuh"
 
+#include <algorithm>
 #include <cstring>
 
 namespace cl {
@@ -562,6 +562,57 @@ inline unsigned grid_for(int64_t n, int threads) {
 
 size_t table_bytes(int bits, int C) { return (size_t)bits * 8 + (size_t)bits * C * 16; }
 
+// The workspace of cl_hdr_merge: cl_hdr_merge_workspace_bytes reports `total`, cl_hdr_merge carves these offsets.
+//   [0, tables)         more than 256 DN rows: the generic kernel's tables or the 16-bit kernel's interleaved rows,
+//                       whichever runs (sized for the larger)
+//   [counts, list)      8-bit C = 3 / 1 stacks unless algo = 1: per-tile bad-pixel bucket counts {count, pad x3}
+//   [list, entries)     the work list, right behind the counts so that one memset clears both: kHotListHeader
+//                       words (hot_list[0] counts the entries) and hot_cap entries, padded to 16 bytes
+//   [entries, end)      per-tile bucket entries {meta, pad, sigma}, 16-byte aligned for the bulk copies
+// `total` reserves the whole 16 bytes the padding can take.
+struct MergeWorkspace {
+    size_t tables = 0, counts = 0, list = 0, entries = 0, end = 0, total = 0;
+    size_t hot_cap = 0;
+    int64_t n_full_tiles = 0;
+};
+
+MergeWorkspace merge_workspace(const cl_hdr_merge_args& a) {
+    MergeWorkspace w;
+    if (a.bits > 256)
+        w.tables = std::max(table_bytes(a.bits, a.channels), wide_table_bytes(a.bits, a.channels, a.std_lut != nullptr));
+    w.counts = w.list = w.entries = w.end = w.total = w.tables;
+    if (a.dn_bytes == 1 && (a.channels == 3 || a.channels == 1) && a.algo != 1) {
+        const int64_t n = (int64_t)a.height * a.width * a.channels;
+        w.n_full_tiles = n / (kStagedTilePx * 3);
+        w.hot_cap = (size_t)std::max<int64_t>(n / 16, 65536);
+        const size_t entries_bytes = (size_t)w.n_full_tiles * kBucketCap * 16;
+        w.list = w.counts + (size_t)w.n_full_tiles * 16;
+        const size_t list_end = w.list + (kHotListHeader + w.hot_cap) * sizeof(uint32_t);
+        w.entries = (list_end + 15) / 16 * 16;
+        w.end = w.entries + entries_bytes;
+        w.total = list_end + 16 + entries_bytes;
+    }
+    return w;
+}
+
+// generic kernel: any stack; its tables are built in shared memory, or (more than 256 DN rows) in the workspace
+int try_merge_generic(MergeParams p, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+    const bool tab_smem = p.bits <= 256;
+    if (!tab_smem) {
+        if (!workspace || workspace_bytes < table_bytes(p.bits, p.C)) return CL_ERR_WORKSPACE;
+        if (!aligned(workspace, 16)) return CL_ERR_ALIGNMENT;
+        double* wt = reinterpret_cast<double*>(workspace);
+        double2* pb = reinterpret_cast<double2*>(wt + p.bits);
+        build_tables_kernel<<<(p.bits + 255) / 256, 256, 0, stream>>>(p.lut, p.dlut, p.max_dn, p.bits, p.C, wt, pb);
+        const int st = launched();
+        if (st != CL_OK) return st;
+        p.g_wt = wt;
+        p.g_pb = pb;
+    }
+    return p.max_dn == 255.0 ? launch_generic<uint8_t>(p, tab_smem, 0, stream)
+                             : launch_generic<uint16_t>(p, tab_smem, 0, stream);
+}
+
 }  // namespace
 
 int launch_merge_generic_range(const MergeParams& p, int64_t first_item, cudaStream_t stream) {
@@ -581,10 +632,6 @@ int launch_dark_scan(const MergeParams& p, cudaStream_t stream) {
     return launched();
 }
 
-size_t bucket_bytes(int64_t n_pixels) {
-    return (size_t)(n_pixels / kStagedTilePx) * kBucketWords * sizeof(uint32_t);
-}
-
 int clear_hot_list(const MergeParams& p, cudaStream_t stream) {
     return cuda_status(cudaMemsetAsync(p.hot_list, 0, kHotListHeader * sizeof(uint32_t), stream));
 }
@@ -594,36 +641,38 @@ int launch_merge_fixup(const MergeParams& p, cudaStream_t stream) {
     return launched();
 }
 
-size_t hot_list_entries(int64_t n_samples) {
-    int64_t cap = n_samples / 16;
-    if (cap < 65536) cap = 65536;
-    return (size_t)cap;
-}
-
 }  // namespace cl
 
 extern "C" {
 
 size_t cl_hdr_merge_workspace_bytes(const cl_hdr_merge_args* a) {
-    if (!a) return 0;
-    size_t bytes = 0;
-    if (a->bits > 256) {                 // generic tables, or the 16-bit kernel's (32-byte rows with an STD table)
-        const size_t generic = cl::table_bytes(a->bits, a->channels);
-        const size_t wide = cl::wide_table_bytes(a->bits, a->channels, a->std_lut != nullptr);
-        bytes += generic > wide ? generic : wide;
-    }
-    // work list (bad pixels whose tile bucket overflowed; samples the single-pass kernel hands to the exact two-pass
-    // formula) + per-tile bad-pixel buckets of the 8-bit RGB / mono fast kernels
-    if (a->dn_bytes == 1 && (a->channels == 3 || a->channels == 1) && a->algo != 1)
-        bytes += (cl::kHotListHeader + cl::hot_list_entries((int64_t)a->height * a->width * a->channels)) *
-                     sizeof(uint32_t) +
-                 cl::bucket_bytes((int64_t)a->height * a->width * a->channels / 3) + 16;
-    return bytes;
+    return a ? cl::merge_workspace(*a).total : 0;
 }
 
+// Which kernel runs.  The requested algo names an ordered list of candidates; the first that handles the stack and
+// has its part of the workspace runs, and each is asked once:
+//   algo 0 (auto)   16-bit, single-pass, single-pass STD-table, staged, staged STD-table, generic
+//   algo 1          generic
+//   algo 2          staged, staged STD-table
+//   algo 3          16-bit
+//   algo 4          single-pass, single-pass STD-table
+//
+//   candidate                                handles                                        workspace
+//   16-bit (hdr_merge_wide.cu)               uint16, N <= 16: the pipelined kernel when     32-byte-aligned table rows
+//                                            every exposure has an uncertainty image or
+//                                            none has, round 1's kernel when they mix
+//   single-pass (hdr_merge_stream.cu)        tile stack, uncertainty images, N >= 2         work list
+//   single-pass STD-table (.._stream_lut.cu) tile stack, STD table, N >= 2                  work list
+//   staged (hdr_merge_staged.cu)             tile stack, uncertainty images                 work list with dark frames
+//   staged STD-table (.._staged_lut.cu)      tile stack, STD table                          work list with dark frames
+//   generic (this file)                      any stack                                      tables above 256 DN rows
+// A tile stack is an 8-bit RGB or mono stack of at least one 512-pixel tile (staged_common.cuh: tile_stack), and the
+// tile kernel's shared-memory layout must fit it.  When no candidate runs, nothing has been enqueued and the call
+// returns CL_ERR_WORKSPACE if a candidate lacked only its workspace, CL_ERR_UNSUPPORTED otherwise.
 int cl_hdr_merge(const cl_hdr_merge_args* a, void* workspace, size_t workspace_bytes, void* stream) {
     using namespace cl;
     CL_REQUIRE(a != nullptr);
+    CL_REQUIRE(a->algo >= 0 && a->algo <= 4);
     CL_REQUIRE(a->n_exposures >= 1 && a->n_exposures <= CL_MAX_EXPOSURES);
     CL_REQUIRE(a->height >= 0 && a->width >= 0 && a->channels >= 1 && a->channels <= CL_MAX_CHANNELS);
     CL_REQUIRE(a->dn_bytes == 1 || a->dn_bytes == 2);
@@ -680,68 +729,43 @@ int cl_hdr_merge(const cl_hdr_merge_args* a, void* workspace, size_t workspace_b
         }
     }
 
-    cudaStream_t s = (cudaStream_t)stream;
-    const bool tab_smem = a->bits <= 256;
-    // 16-bit stacks with uncertainty images and N <= 16: fused-table kernel (hdr_merge_wide.cu)
-    bool wide = false;
-    if (!tab_smem && a->algo != 1 && a->algo != 2 && a->algo != 4) {
-        if (workspace && aligned(workspace, 32) && workspace_bytes >= wide_table_bytes(p.bits, p.C, !all_std))
-            p.g_tab32 = reinterpret_cast<const double2*>(workspace);
-        wide = merge_wide_supported(p, a->dn_bytes, all_std);
-        if (a->algo == 3 && !wide) return p.g_tab32 ? CL_ERR_UNSUPPORTED : CL_ERR_WORKSPACE;
-    } else if (a->algo == 3) {
-        return CL_ERR_UNSUPPORTED;
-    }
-    if (wide) return launch_merge_wide(p, s);
-    if (!tab_smem) {
-        const size_t need = table_bytes(p.bits, p.C);
-        if (!workspace || workspace_bytes < need) return CL_ERR_WORKSPACE;
-        if (!aligned(workspace, 16)) return CL_ERR_ALIGNMENT;
-        double* wt = reinterpret_cast<double*>(workspace);
-        double2* pb = reinterpret_cast<double2*>(wt + p.bits);
-        build_tables_kernel<<<(p.bits + 255) / 256, 256, 0, s>>>(p.lut, p.dlut, p.max_dn, p.bits, p.C,
-                                                                wt, pb);
-        int st = launched();
-        if (st != CL_OK) return st;
-        p.g_wt = wt;
-        p.g_pb = pb;
+    // the workspace, carved as merge_workspace() lays it out
+    const MergeWorkspace ws = merge_workspace(*a);
+    unsigned char* w = static_cast<unsigned char*>(workspace);
+    if (ws.tables && w && aligned(w, 32) && workspace_bytes >= wide_table_bytes(p.bits, p.C, !all_std))
+        p.g_tab32 = reinterpret_cast<const double2*>(w);
+    if (ws.end > ws.counts && w && aligned(w, 16) && workspace_bytes >= ws.end) {
+        p.n_full_tiles = (int32_t)ws.n_full_tiles;
+        p.bucket_counts = reinterpret_cast<uint32_t*>(w + ws.counts);
+        p.hot_list = reinterpret_cast<uint32_t*>(w + ws.list);
+        p.hot_cap = (uint32_t)ws.hot_cap;
+        p.bucket_entries = reinterpret_cast<uint32_t*>(w + ws.entries);
     }
 
-    if (a->dn_bytes == 1 && (p.C == 3 || p.C == 1) && a->algo != 1) {
-        const size_t off = tab_smem ? 0 : table_bytes(p.bits, p.C);
-        const size_t entries = hot_list_entries((int64_t)p.H * p.W * p.C);
-        const size_t list_bytes = ((kHotListHeader + entries) * sizeof(uint32_t) + 15) / 16 * 16;
-        const size_t bkt_bytes = (bucket_bytes((int64_t)p.H * p.W * p.C / 3) + 15) / 16 * 16;
-        if (workspace && aligned(workspace, 16) && workspace_bytes >= off + list_bytes + bkt_bytes) {
-            // [bucket counts][hot-list header + entries][bucket entries]
-            p.n_full_tiles = (int32_t)(((int64_t)p.H * p.W * p.C) / (kStagedTilePx * 3));
-            p.bucket_counts = reinterpret_cast<uint32_t*>(reinterpret_cast<unsigned char*>(workspace) + off);
-            p.hot_list = p.bucket_counts + (size_t)p.n_full_tiles * 4;
-            p.hot_cap = (uint32_t)entries;
-            p.bucket_entries = p.hot_list + list_bytes / sizeof(uint32_t);
-        } else if ((a->algo == 2 && p.any_dark) || a->algo == 4) {
-            return CL_ERR_WORKSPACE;
+    enum Candidate { kWide, kStream, kStreamLut, kStaged, kStagedLut, kGeneric, kEnd };
+    static constexpr Candidate kCandidates[5][7] = {
+        {kWide, kStream, kStreamLut, kStaged, kStagedLut, kGeneric, kEnd},
+        {kGeneric, kEnd},
+        {kStaged, kStagedLut, kEnd},
+        {kWide, kEnd},
+        {kStream, kStreamLut, kEnd},
+    };
+    cudaStream_t s = (cudaStream_t)stream;
+    int status = CL_ERR_UNSUPPORTED;
+    for (const Candidate* c = kCandidates[a->algo]; *c != kEnd; ++c) {
+        int st;
+        switch (*c) {
+            case kWide: st = try_merge_wide(p, s); break;
+            case kStream: st = try_merge_stream(p, s); break;
+            case kStreamLut: st = try_merge_stream_lut(p, s); break;
+            case kStaged: st = try_merge_staged(p, s); break;
+            case kStagedLut: st = try_merge_staged_lut(p, s); break;
+            default: st = try_merge_generic(p, workspace, workspace_bytes, s); break;
         }
+        if (st == CL_ERR_WORKSPACE) status = st;
+        else if (st != CL_ERR_UNSUPPORTED) return st;
     }
-    int algo = a->algo;
-    const bool staged_ok = merge_staged_supported(p, all_std);
-    const bool staged_lut_ok = !staged_ok && merge_staged_lut_supported(p);   // no uncertainty images: STD table
-    const bool stream_ok = merge_stream_supported(p, all_std);                // float64 uncertainty images
-    const bool stream_lut_ok = !stream_ok && merge_stream_lut_supported(p);   // STD table
-    if (algo == 0) algo = (stream_ok || stream_lut_ok) ? 4 : (staged_ok || staged_lut_ok) ? 2 : 1;
-    if (algo == 4) {                   // single-pass kernels (expanded variance, see hdr_merge_stream.cu)
-        if (stream_ok) return launch_merge_stream(p, s);
-        if (stream_lut_ok) return launch_merge_stream_lut(p, s);
-        return CL_ERR_UNSUPPORTED;
-    }
-    if (algo == 2) {
-        if (staged_lut_ok) return launch_merge_staged_lut(p, s);
-        if (!staged_ok) return CL_ERR_UNSUPPORTED;
-        return launch_merge_staged(p, s);
-    }
-    if (algo != 1) return CL_ERR_INVALID_ARGUMENT;
-    if (a->dn_bytes == 1) return launch_generic<uint8_t>(p, tab_smem, 0, s);
-    return launch_generic<uint16_t>(p, tab_smem, 0, s);
+    return status;
 }
 
 size_t cl_flat_roi_means_workspace_bytes(int height, int width, int channels) {

@@ -1,7 +1,7 @@
 // K2 shared definitions: kernel parameter block, per-exposure accumulation, median replace and
-// the flat-field epilogue, used by both HDR-merge kernels (generic register kernel and the
-// bulk-copy staged kernel).  The two kernels run the same arithmetic in the same order, so their
-// outputs are bit-identical (tests/test_gpu_hdr_merge.py checks that).
+// the flat-field epilogue, used by every HDR-merge kernel.  The two-pass kernels run the same
+// arithmetic in the same order, so their outputs are bit-identical; the single-pass kernels'
+// expanded variance is checked against them (tests/test_gpu_hdr_merge.py).
 #pragma once
 
 #include "common.cuh"
@@ -339,17 +339,15 @@ __device__ __noinline__ void recompute_sample(const MergeParams& p, int64_t i) {
     p.out_std[i] = os;
 }
 
-int launch_merge_staged(const MergeParams& p, cudaStream_t stream);   // hdr_merge_staged.cu
-int launch_merge_stream(const MergeParams& p, cudaStream_t stream);   // hdr_merge_stream.cu
-bool merge_stream_supported(const MergeParams& p, bool all_std_images);
-int launch_merge_stream_lut(const MergeParams& p, cudaStream_t stream);   // hdr_merge_stream_lut.cu
-bool merge_stream_lut_supported(const MergeParams& p);
-int launch_merge_staged_lut(const MergeParams& p, cudaStream_t stream);   // hdr_merge_staged_lut.cu
-bool merge_staged_lut_supported(const MergeParams& p);
-int launch_merge_wide(const MergeParams& p, cudaStream_t stream);     // hdr_merge_wide.cu
-bool merge_wide_supported(const MergeParams& p, int dn_bytes, bool all_std_images);
-size_t wide_table_bytes(int bits, int C, bool with_std_lut);
-bool merge_staged_supported(const MergeParams& p, bool all_std_images);
+// One "try" per kernel family (the selection table is in hdr_merge.cu): CL_ERR_UNSUPPORTED when the kernel does not
+// handle the stack, CL_ERR_WORKSPACE when only its part of the workspace is missing -- both before anything is
+// enqueued -- otherwise the status of its launches.
+int try_merge_wide(const MergeParams& p, cudaStream_t stream);         // hdr_merge_wide.cu
+int try_merge_stream(const MergeParams& p, cudaStream_t stream);       // hdr_merge_stream.cu
+int try_merge_stream_lut(const MergeParams& p, cudaStream_t stream);   // hdr_merge_stream_lut.cu
+int try_merge_staged(const MergeParams& p, cudaStream_t stream);       // hdr_merge_staged.cu
+int try_merge_staged_lut(const MergeParams& p, cudaStream_t stream);   // hdr_merge_staged_lut.cu
+size_t wide_table_bytes(int bits, int C, bool with_std_lut);            // hdr_merge_wide.cu
 // hdr_merge.cu
 int launch_merge_generic_range(const MergeParams& p, int64_t first_item, cudaStream_t stream);
 int launch_dark_scan(const MergeParams& p, cudaStream_t stream);

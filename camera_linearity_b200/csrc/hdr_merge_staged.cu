@@ -334,53 +334,14 @@ bool make_layout(const MergeParams& p, StagedLayout& L) {
 
 }  // namespace
 
-bool merge_staged_supported(const MergeParams& p, bool all_std_images) {
-    if ((p.C != kC && p.C != 1) || p.bits != 256 || p.max_dn != 255.0 || !all_std_images) return false;
-    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
-    if (n_samples < kTilePx * kC || n_samples >= 0xFFFFFFFFll) return false;
-    if (p.any_dark && (!p.hot_list || p.hot_cap == 0 || !p.bucket_counts || !p.bucket_entries)) return false;
-    if (p.flat_bytes && (!aligned(p.flat_std, 16) || !aligned(p.flat, 16))) return false;
+int try_merge_staged(const MergeParams& p, cudaStream_t stream) {
     StagedLayout L;
-    return make_layout(p, L);
-}
-
-int launch_merge_staged(const MergeParams& p, cudaStream_t stream) {
-    StagedLayout L;
-    if (!make_layout(p, L)) return CL_ERR_UNSUPPORTED;
-    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
-    const int n_tiles = (int)(n_samples / (kTilePx * kC));
-    int grid = sm_count();
-    if (grid > n_tiles) grid = n_tiles;
-    auto launch = [&](auto kernel) -> int {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)L.total);
-        if (e != cudaSuccess) return cuda_status(e);
-        kernel<<<grid, kThreads, L.total, stream>>>(p, L, n_tiles);
-        return launched();
-    };
-    int st;
-    if (p.any_dark) {                 // work list of bad samples for the fix-up pass
-        st = launch_dark_scan(p, stream);
-        if (st != CL_OK) return st;
-    }
-    if (p.C == 1) {
-        if (p.n <= 8) st = launch(merge_staged_kernel<8, true>);
-        else if (p.n <= 16) st = launch(merge_staged_kernel<16, true>);
-        else st = launch(merge_staged_kernel<32, true>);
-    } else {
-        if (p.n <= 8) st = launch(merge_staged_kernel<8, false>);
-        else if (p.n <= 16) st = launch(merge_staged_kernel<16, false>);
-        else st = launch(merge_staged_kernel<32, false>);
-    }
-    if (st != CL_OK) return st;
-    // pixels past the last full tile (< 512) go through the generic kernel; both kernels run
-    // identical arithmetic, so the seam is invisible
-    const int64_t tail_first_sample = (int64_t)n_tiles * kTilePx * kC;
-    if (tail_first_sample < n_samples) {
-        st = launch_merge_generic_range(p, tail_first_sample / 4, stream);
-        if (st != CL_OK) return st;
-    }
-    return p.any_dark ? launch_merge_fixup(p, stream) : CL_OK;
+    if (!tile_stack(p, true) || !make_layout(p, L)) return CL_ERR_UNSUPPORTED;
+    const bool mono = p.C == 1;
+    auto kernel = p.n <= 8    ? (mono ? merge_staged_kernel<8, true> : merge_staged_kernel<8, false>)
+                  : p.n <= 16 ? (mono ? merge_staged_kernel<16, true> : merge_staged_kernel<16, false>)
+                              : (mono ? merge_staged_kernel<32, true> : merge_staged_kernel<32, false>);
+    return launch_tile_kernel(p, kernel, kThreads, L, stream);
 }
 
 }  // namespace cl

@@ -235,50 +235,13 @@ bool make_lut_layout(const MergeParams& p, LutLayout& L) {
 
 }  // namespace
 
-bool merge_staged_lut_supported(const MergeParams& p) {
-    if ((p.C != kC && p.C != 1) || p.bits != 256 || p.max_dn != 255.0 || !p.std_lut) return false;
-    for (int k = 0; k < p.n; ++k)
-        if (p.std[k]) return false;                   // mixed images / table: generic kernel
-    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
-    if (n_samples < kTilePx * kC || n_samples >= 0xFFFFFFFFll) return false;
-    if (p.any_dark && (!p.hot_list || p.hot_cap == 0 || !p.bucket_counts || !p.bucket_entries)) return false;
-    if (p.flat_bytes && (!aligned(p.flat_std, 8) || !aligned(p.flat, 16))) return false;
+int try_merge_staged_lut(const MergeParams& p, cudaStream_t stream) {
     LutLayout L;
-    return make_lut_layout(p, L);
-}
-
-int launch_merge_staged_lut(const MergeParams& p, cudaStream_t stream) {
-    LutLayout L;
-    if (!make_lut_layout(p, L)) return CL_ERR_UNSUPPORTED;
-    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
-    const int n_tiles = (int)(n_samples / (kTilePx * kC));
-    int grid = sm_count();
-    if (grid > n_tiles) grid = n_tiles;
-    auto launch = [&](auto kernel) -> int {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
-        if (e != cudaSuccess) return cuda_status(e);
-        kernel<<<grid, kThreads, L.total, stream>>>(p, L, n_tiles);
-        return launched();
-    };
-    int st;
-    if (p.any_dark) {
-        st = launch_dark_scan(p, stream);
-        if (st != CL_OK) return st;
-    }
-    if (p.C == 1) {
-        if (p.n <= 8) st = launch(merge_staged_lut_kernel<8, true>);
-        else st = launch(merge_staged_lut_kernel<16, true>);
-    } else {
-        if (p.n <= 8) st = launch(merge_staged_lut_kernel<8, false>);
-        else st = launch(merge_staged_lut_kernel<16, false>);
-    }
-    if (st != CL_OK) return st;
-    const int64_t tail_first_sample = (int64_t)n_tiles * kTilePx * kC;
-    if (tail_first_sample < n_samples) {
-        st = launch_merge_generic_range(p, tail_first_sample / 4, stream);
-        if (st != CL_OK) return st;
-    }
-    return p.any_dark ? launch_merge_fixup(p, stream) : CL_OK;
+    if (!tile_stack(p, false) || !make_lut_layout(p, L)) return CL_ERR_UNSUPPORTED;
+    const bool mono = p.C == 1;
+    auto kernel = p.n <= 8 ? (mono ? merge_staged_lut_kernel<8, true> : merge_staged_lut_kernel<8, false>)
+                           : (mono ? merge_staged_lut_kernel<16, true> : merge_staged_lut_kernel<16, false>);
+    return launch_tile_kernel(p, kernel, kThreads, L, stream);
 }
 
 }  // namespace cl

@@ -266,13 +266,8 @@ merge_stream_kernel(const __grid_constant__ MergeParams p, const StreamLayout L,
             // calls they replace, without the six range tests + slow-path branches per pixel that fenced the
             // epilogue's schedule.  A sample that is off a main path joins the cancelled ones on the work list
             // (merge_fixup_kernel recomputes it with the library calls).
-#ifndef CL_STREAM_LIBRARY_MATH
             bool k0, k1, k2;
             const double r0 = rcp_main_path(S0, k0), r1 = rcp_main_path(S1, k1), r2 = rcp_main_path(S2, k2);
-#else
-            const bool k0 = true, k1 = true, k2 = true;
-            const double r0 = 1.0 / S0, r1 = 1.0 / S1, r2 = 1.0 / S2;
-#endif
             double v0 = av0 * r0, v1 = av1 * r1, v2 = av2 * r2;
             const double q0 = expanded_variance(A0, B0, C0, r0), q1 = expanded_variance(A1, B1, C1, r1),
                          q2 = expanded_variance(A2, B2, C2, r2);
@@ -297,27 +292,17 @@ merge_stream_kernel(const __grid_constant__ MergeParams p, const StreamLayout L,
                     rf2 = flat_recip(p.flat, p.flat_bytes, i0 + 2, p.max_dn);
                 }
                 constexpr int c1 = MONO ? 0 : 1, c2 = MONO ? 0 : 2;
-#ifndef CL_STREAM_LIBRARY_MATH
                 f0 |= !flat_apply_main_path(v0, u0, (q0 * r0) * r0, rf0, fs0, p.flat_means[0], p.flat_means[kCt + 0]);
                 f1 |= !flat_apply_main_path(v1, u1, (q1 * r1) * r1, rf1, fs1, p.flat_means[c1], p.flat_means[kCt + c1]);
                 f2 |= !flat_apply_main_path(v2, u2, (q2 * r2) * r2, rf2, fs2, p.flat_means[c2], p.flat_means[kCt + c2]);
-#else
-                flat_apply(v0, u0, (q0 * r0) * r0, rf0, fs0, p.flat_means[0], p.flat_means[kCt + 0]);
-                flat_apply(v1, u1, (q1 * r1) * r1, rf1, fs1, p.flat_means[c1], p.flat_means[kCt + c1]);
-                flat_apply(v2, u2, (q2 * r2) * r2, rf2, fs2, p.flat_means[c2], p.flat_means[kCt + c2]);
-#endif
                 __syncwarp();
                 if (lane == 0 && consumed(u0, u1, u2 + rf0)) mbar_arrive(&empty[s]);     // (rf: the staged flat bytes)
                 if (++s == stages) { s = 0; phase ^= 1; }
             } else {
-#ifndef CL_STREAM_LIBRARY_MATH
                 bool s0, s1, s2;
                 const double t0 = sqrt_main_path(q0, s0), t1 = sqrt_main_path(q1, s1), t2 = sqrt_main_path(q2, s2);
                 u0 = (s0 ? t0 : 0.0) * r0; u1 = (s1 ? t1 : 0.0) * r1; u2 = (s2 ? t2 : 0.0) * r2;
                 f0 |= !(s0 || q0 == 0.0); f1 |= !(s1 || q1 == 0.0); f2 |= !(s2 || q2 == 0.0);
-#else
-                u0 = sqrt(q0) * r0; u1 = sqrt(q1) * r1; u2 = sqrt(q2) * r2;
-#endif
             }
             // samples whose expansion cancelled (or that left a main path) go to the exact formula (work list ->
             // merge_fixup_kernel); one atomic per warp and channel that has any
@@ -350,41 +335,13 @@ bool make_stream_layout(StreamLayout& L) {
 
 }  // namespace
 
-bool merge_stream_supported(const MergeParams& p, bool all_std_images) {
-    if ((p.C != kC && p.C != 1) || p.bits != 256 || p.max_dn != 255.0 || !all_std_images || p.n < 2) return false;
-    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
-    if (n_samples < kTilePx * kC || n_samples >= 0xFFFFFFFFll) return false;
-    if (!p.hot_list || p.hot_cap == 0 || !p.bucket_counts || !p.bucket_entries) return false;
-    if (p.flat_bytes && (!aligned(p.flat_std, 16) || !aligned(p.flat, 16))) return false;
+int try_merge_stream(const MergeParams& p_in, cudaStream_t stream) {
     StreamLayout L;
-    return make_stream_layout(L);
-}
-
-int launch_merge_stream(const MergeParams& p_in, cudaStream_t stream) {
+    if (!tile_stack(p_in, true) || p_in.n < 2 || !make_stream_layout(L)) return CL_ERR_UNSUPPORTED;
     MergeParams p = p_in;
     p.stream_mode = 1;
-    StreamLayout L;
-    if (!make_stream_layout(L)) return CL_ERR_UNSUPPORTED;
-    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
-    const int n_tiles = (int)(n_samples / (kTilePx * kC));
-    int grid = sm_count();
-    if (grid > n_tiles) grid = n_tiles;
-    auto launch = [&](auto kernel) -> int {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
-        if (e != cudaSuccess) return cuda_status(e);
-        kernel<<<grid, kThreads, L.total, stream>>>(p, L, n_tiles);
-        return launched();
-    };
-    int st = p.any_dark ? launch_dark_scan(p, stream) : clear_hot_list(p, stream);     // (the scan clears the list too)
-    if (st != CL_OK) return st;
-    st = p.C == 1 ? launch(merge_stream_kernel<true>) : launch(merge_stream_kernel<false>);
-    if (st != CL_OK) return st;
-    const int64_t tail_first_sample = (int64_t)n_tiles * kTilePx * kC;
-    if (tail_first_sample < n_samples) {
-        st = launch_merge_generic_range(p, tail_first_sample / 4, stream);
-        if (st != CL_OK) return st;
-    }
-    return launch_merge_fixup(p, stream);       // bucket overflows and cancelled samples (usually an empty list)
+    return launch_tile_kernel(p, p.C == 1 ? merge_stream_kernel<true> : merge_stream_kernel<false>, kThreads, L,
+                              stream);
 }
 
 }  // namespace cl

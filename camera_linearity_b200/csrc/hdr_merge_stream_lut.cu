@@ -251,13 +251,8 @@ merge_stream_lut_kernel(const __grid_constant__ MergeParams p, const SLutLayout 
             }
             // 1 / S and the square roots: the library's main paths (see merge_stream_kernel); a sample off them joins
             // the cancelled ones on the work list
-#ifndef CL_STREAM_LIBRARY_MATH
             bool k0, k1, k2;
             const double r0 = rcp_main_path(S0, k0), r1 = rcp_main_path(S1, k1), r2 = rcp_main_path(S2, k2);
-#else
-            const bool k0 = true, k1 = true, k2 = true;
-            const double r0 = 1.0 / S0, r1 = 1.0 / S1, r2 = 1.0 / S2;
-#endif
             double v0 = av0 * r0, v1 = av1 * r1, v2 = av2 * r2;
             const double q0 = expanded_variance(A0, B0, C0, r0), q1 = expanded_variance(A1, B1, C1, r1),
                          q2 = expanded_variance(A2, B2, C2, r2);
@@ -282,24 +277,14 @@ merge_stream_lut_kernel(const __grid_constant__ MergeParams p, const SLutLayout 
                     rf2 = flat_recip(p.flat, p.flat_bytes, i0 + 2, p.max_dn);
                 }
                 constexpr int c1 = MONO ? 0 : 1, c2 = MONO ? 0 : 2;
-#ifndef CL_STREAM_LIBRARY_MATH
                 c0 |= !flat_apply_main_path(v0, u0, (q0 * r0) * r0, rf0, f0, p.flat_means[0], p.flat_means[kCt + 0]);
                 c1f |= !flat_apply_main_path(v1, u1, (q1 * r1) * r1, rf1, f1, p.flat_means[c1], p.flat_means[kCt + c1]);
                 c2f |= !flat_apply_main_path(v2, u2, (q2 * r2) * r2, rf2, f2, p.flat_means[c2], p.flat_means[kCt + c2]);
-#else
-                flat_apply(v0, u0, (q0 * r0) * r0, rf0, f0, p.flat_means[0], p.flat_means[kCt + 0]);
-                flat_apply(v1, u1, (q1 * r1) * r1, rf1, f1, p.flat_means[c1], p.flat_means[kCt + c1]);
-                flat_apply(v2, u2, (q2 * r2) * r2, rf2, f2, p.flat_means[c2], p.flat_means[kCt + c2]);
-#endif
             } else {
-#ifndef CL_STREAM_LIBRARY_MATH
                 bool s0, s1, s2;
                 const double t0 = sqrt_main_path(q0, s0), t1 = sqrt_main_path(q1, s1), t2 = sqrt_main_path(q2, s2);
                 u0 = (s0 ? t0 : 0.0) * r0; u1 = (s1 ? t1 : 0.0) * r1; u2 = (s2 ? t2 : 0.0) * r2;
                 c0 |= !(s0 || q0 == 0.0); c1f |= !(s1 || q1 == 0.0); c2f |= !(s2 || q2 == 0.0);
-#else
-                u0 = sqrt(q0) * r0; u1 = sqrt(q1) * r1; u2 = sqrt(q2) * r2;
-#endif
             }
             // samples whose expansion cancelled (or that left a main path) go to the exact formula (work list ->
             // merge_fixup_kernel)
@@ -332,43 +317,13 @@ bool make_slut_layout(SLutLayout& L) {
 
 }  // namespace
 
-bool merge_stream_lut_supported(const MergeParams& p) {
-    if ((p.C != kC && p.C != 1) || p.bits != 256 || p.max_dn != 255.0 || !p.std_lut || p.n < 2) return false;
-    for (int k = 0; k < p.n; ++k)
-        if (p.std[k]) return false;                   // mixed images / table: two-pass kernels
-    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
-    if (n_samples < kTilePx * kC || n_samples >= 0xFFFFFFFFll) return false;
-    if (!p.hot_list || p.hot_cap == 0 || !p.bucket_counts || !p.bucket_entries) return false;
-    if (p.flat_bytes && (!aligned(p.flat_std, 8) || !aligned(p.flat, 16))) return false;
+int try_merge_stream_lut(const MergeParams& p_in, cudaStream_t stream) {
     SLutLayout L;
-    return make_slut_layout(L);
-}
-
-int launch_merge_stream_lut(const MergeParams& p_in, cudaStream_t stream) {
+    if (!tile_stack(p_in, false) || p_in.n < 2 || !make_slut_layout(L)) return CL_ERR_UNSUPPORTED;
     MergeParams p = p_in;
     p.stream_mode = 2;
-    SLutLayout L;
-    if (!make_slut_layout(L)) return CL_ERR_UNSUPPORTED;
-    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
-    const int n_tiles = (int)(n_samples / (kTilePx * kC));
-    int grid = sm_count();
-    if (grid > n_tiles) grid = n_tiles;
-    auto launch = [&](auto kernel) -> int {
-        cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
-        if (e != cudaSuccess) return cuda_status(e);
-        kernel<<<grid, kThreads, L.total, stream>>>(p, L, n_tiles);
-        return launched();
-    };
-    int st = p.any_dark ? launch_dark_scan(p, stream) : clear_hot_list(p, stream);     // (the scan clears the list too)
-    if (st != CL_OK) return st;
-    st = p.C == 1 ? launch(merge_stream_lut_kernel<true>) : launch(merge_stream_lut_kernel<false>);
-    if (st != CL_OK) return st;
-    const int64_t tail_first_sample = (int64_t)n_tiles * kTilePx * kC;
-    if (tail_first_sample < n_samples) {
-        st = launch_merge_generic_range(p, tail_first_sample / 4, stream);
-        if (st != CL_OK) return st;
-    }
-    return launch_merge_fixup(p, stream);       // bucket overflows, table mismatches, cancelled samples
+    return launch_tile_kernel(p, p.C == 1 ? merge_stream_lut_kernel<true> : merge_stream_lut_kernel<false>, kThreads,
+                              L, stream);
 }
 
 }  // namespace cl

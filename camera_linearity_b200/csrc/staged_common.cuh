@@ -1,7 +1,9 @@
-// mbarrier / bulk-copy (TMA 1-D) PTX wrappers and the data-dependent stage-release predicates shared by the
-// two staged HDR-merge kernels (hdr_merge_staged.cu: float64 uncertainty images through a shared-memory ring;
-// hdr_merge_staged_lut.cu: uncertainties from the camera's STD table).
+// mbarrier / bulk-copy (TMA 1-D) PTX wrappers, the data-dependent stage-release predicates, and the stack test and
+// launch sequence shared by the four 8-bit tile kernels (hdr_merge_staged.cu, hdr_merge_staged_lut.cu,
+// hdr_merge_stream.cu, hdr_merge_stream_lut.cu).
 #pragma once
+
+#include <algorithm>
 
 #include "hdr_merge.cuh"
 
@@ -69,6 +71,49 @@ __device__ __forceinline__ bool consumed_nonneg(double a, double b, double c) {
     return m + 0x00100000u < 0x80100000u;
 }
 
+// What every tile kernel needs of the stack: 8-bit DNs (256-row tables), C = 3 or 1 (mono runs as virtual RGB), at
+// least one full 512-pixel tile, 32-bit sample indices, and the uncertainty of every exposure from an image
+// (std_images) or of none (the STD table).  The flat's DN bytes are bulk-copied; its uncertainties are too when the
+// kernel streams uncertainty images, the STD-table kernels load them per sample.
+inline bool tile_stack(const MergeParams& p, bool std_images) {
+    if ((p.C != 3 && p.C != 1) || p.bits != 256) return false;
+    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
+    if (n_samples < kStagedTilePx * 3 || n_samples >= 0xFFFFFFFFll) return false;
+    if (!std_images && !p.std_lut) return false;
+    for (int k = 0; k < p.n; ++k)
+        if ((p.std[k] != nullptr) != std_images) return false;
+    return !p.flat_bytes || (aligned(p.flat, 16) && aligned(p.flat_std, std_images ? 16 : 8));
+}
+
+// The launch sequence of a tile kernel: [dark scan | work-list clear], the kernel on the full tiles (one CTA per SM, at
+// most one per tile), the generic kernel on the ragged tail, [fix-up].  The single-pass kernels (p.stream_mode != 0)
+// also file cancelled samples in the work list, so they always clear or fill it and always run the fix-up; the
+// two-pass kernels use it only for the bad pixels of dark frames.  CL_ERR_WORKSPACE, with nothing enqueued, when the
+// sequence needs the work list and the workspace held none.
+template <typename Layout>
+int launch_tile_kernel(const MergeParams& p, void (*kernel)(MergeParams, Layout, int), int threads, const Layout& L,
+                       cudaStream_t stream) {
+    const bool single_pass = p.stream_mode != 0;
+    if ((single_pass || p.any_dark) && !p.hot_list) return CL_ERR_WORKSPACE;
+    const int64_t n_samples = (int64_t)p.H * p.W * p.C;
+    const int n_tiles = (int)(n_samples / (kStagedTilePx * 3));
+    int st = CL_OK;
+    if (p.any_dark) st = launch_dark_scan(p, stream);           // (the scan clears the list too)
+    else if (single_pass) st = clear_hot_list(p, stream);
+    if (st != CL_OK) return st;
+    const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total);
+    if (e != cudaSuccess) return cuda_status(e);
+    kernel<<<std::min(sm_count(), n_tiles), threads, L.total, stream>>>(p, L, n_tiles);
+    st = launched();
+    if (st != CL_OK) return st;
+    // pixels past the last full tile (< 512) go through the generic kernel; both kernels run identical arithmetic
+    const int64_t tail_first_sample = (int64_t)n_tiles * kStagedTilePx * 3;
+    if (tail_first_sample < n_samples) {
+        st = launch_merge_generic_range(p, tail_first_sample / 4, stream);
+        if (st != CL_OK) return st;
+    }
+    return single_pass || p.any_dark ? launch_merge_fixup(p, stream) : CL_OK;
+}
 
 }  // namespace staged
 }  // namespace cl
