@@ -12,10 +12,11 @@
 //   unweighted: count, sum(v);
 //   and, for the variance sum(w*(v-mean)^2), the SHIFTED moments T0 = sum(w), T1 = sum(w*d), T2 = sum(w*d^2)
 //   with d = v - K over the samples the variance counts:  sum(w*(v-mean)^2) = T2 - 2(mean-K) T1 + (mean-K)^2 T0.
-// K (per channel, abs and rel) is the plain mean of the first few thousand samples -- every block derives it
-// from the same L2-hot chunk in the same order, so it is one number and costs no launch; with K within a few
-// standard errors of the mean the expansion loses nothing (round 1 made a second pass over the inputs, 64 B
-// per sample, only to centre the variance).  Block partials are combined in a fixed order (deterministic); the
+// K (per channel, abs and rel) is the plain mean of the samples the variance counts in the first of a few chunks of a
+// few thousand samples (the image's first, then chunks spread over the image) that holds one -- every block derives
+// it from the same L2-hot chunks in the same order, so it is one number and costs no launch; with K within a few
+// standard errors of the mean the expansion loses nothing (round 1 made a second pass over the inputs, 64 B per
+// sample, only to centre the variance).  Block partials are combined in a fixed order (deterministic); the
 // reference's pairwise summation differs at the 1e-13 level.
 #include <math.h>
 
@@ -28,7 +29,10 @@ constexpr int kThreads = 256;
 constexpr int kBlocks = 296;  // 148 SMs x 2 resident CTAs; fixed (not sm_count) so the summation order is machine-independent
 constexpr int kQ1 = 8;    // sums per channel: {sw, svw, ssig, nsig} x {abs, rel}
 constexpr int kQ = 14;    // + the shifted moments {T0, T1, T2} x {abs, rel}
-constexpr int kShiftSamples = 16;   // per thread: the provisional mean K comes from the first 16 * lanes_used samples
+constexpr int kShiftSamples = 16;   // per thread: the provisional mean K comes from a chunk of 16 * lanes_used samples
+constexpr int kShiftChunks = 8;     // chunks, at j/8 of the image, scanned for one the variance counts a sample of
+                                    // before K falls back to 0: a channel with no such sample (thresholded away) costs
+                                    // each thread 8 * 16 extra samples
 
 struct PairArgs {
     const double* x_val;
@@ -36,6 +40,8 @@ struct PairArgs {
     const double* y_val;
     const double* y_std;
     double multiplier;
+    double t2_multiplier;    // the m of the general routine's rcp * m: 1 when m = 0, so that sigma_y*x / (m*y*y) is +-inf
+                             // there as in NumPy, not inf * 0 = NaN (the lean routine never runs with m = 0)
     double lower[CL_MAX_CHANNELS], upper[CL_MAX_CHANNELS];
     int has_thr;
     int64_t n;
@@ -45,6 +51,7 @@ struct PairArgs {
 struct Diff {
     double a, r, sa, sr;     // absolute / relative difference and their uncertainties
     double wa, wr;           // 1/sa, 1/sr
+    double qa, qr;           // sa^2, sr^2
     bool bad_v, bad_sa, bad_sr;   // the reference's value would be NaN here (thresholded or NaN input)
 };
 
@@ -81,7 +88,7 @@ __device__ __forceinline__ Diff difference(const PairArgs& p, const Raw& raw, do
     d.a = __dsub_rn(x, scale);
     d.r = __dmul_rn(d.a, inv);
     d.bad_v = nx || ny;
-    d.sa = d.sr = d.wa = d.wr = 0.0;
+    d.sa = d.sr = d.wa = d.wr = d.qa = d.qr = 0.0;
     d.bad_sa = d.bad_sr = false;
     if (use_std) {                                       // :652-653
         const double inf = __longlong_as_double(0x7ff0000000000000LL);
@@ -90,12 +97,14 @@ __device__ __forceinline__ Diff difference(const PairArgs& p, const Raw& raw, do
         d.wa = rsqrt(qa);                                // weights = 1 / stds
         d.sa = (qa > 0.0 && qa < inf) ? __dmul_rn(qa, d.wa) : qa;
         const double t1 = __dmul_rn(xs, inv);
-        const double t2 = __dmul_rn(__dmul_rn(__dmul_rn(ys, x), inv), __dmul_rn(inv, p.multiplier));   // ys*x / (m*y*y)
+        const double t2 = __dmul_rn(__dmul_rn(__dmul_rn(ys, x), inv), __dmul_rn(inv, p.t2_multiplier));   // ys*x / (m*y*y)
         const double qr = __dadd_rn(__dmul_rn(t1, t1), __dmul_rn(t2, t2));
         d.wr = rsqrt(qr);
         d.sr = (qr > 0.0 && qr < inf) ? __dmul_rn(qr, d.wr) : qr;
         d.bad_sa = nxs || nys;
         d.bad_sr = nxs || nys || nx || ny;
+        d.qa = qa;
+        d.qr = qr;
     }
     return d;
 }
@@ -126,10 +135,14 @@ __device__ __forceinline__ void accumulate_shifted(double (&acc)[kQ], const Diff
     double wa = 1.0, wr = 1.0;
     bool bad_a = d.bad_v, bad_r = d.bad_v;
     if (USE_STD) {
+        // An infinite value makes the weighted mean infinite (or NaN), and then its own term (inf - mean)^2 is NaN
+        // in np.nansum: leaving it out keeps T0 the weight of the samples with finite values, which decides
+        // whether the variance about an infinite mean is inf or 0.  With a finite mean no such sample exists.
+        const double inf = __longlong_as_double(0x7ff0000000000000LL);
         wa = d.wa;
         wr = d.wr;
-        bad_a = bad_a || d.bad_sa;
-        bad_r = d.bad_sr;
+        bad_a = bad_a || d.bad_sa || !(fabs(d.a) < inf);
+        bad_r = d.bad_sr || !(fabs(d.r) < inf);
     }
     const double ta = __dmul_rn(wa, __dmul_rn(da, da)), tr = __dmul_rn(wr, __dmul_rn(dr, dr));
     if (!bad_a && not_nan(ta)) { acc[8] += wa; acc[9] = fma(wa, da, acc[9]); acc[10] += ta; }
@@ -248,29 +261,47 @@ pair_stats_kernel(const PairArgs p, double* __restrict__ partial /* [blocks][kQ]
     const bool active = (int)threadIdx.x < lanes_used;
     const int c = threadIdx.x % C;                           // (block offset and stride are multiples of C)
     const double lo = p.lower[c], hi = p.upper[c];
-    // ---- provisional means K from the first kShiftSamples * lanes_used samples (identical in every block) ----
+    // ---- provisional means K (identical in every block) ----
+    // K is the plain mean of the samples the variance counts -- a finite value and, with uncertainty images, a finite
+    // positive weight -- in the first chunk of kShiftSamples * lanes_used samples that holds one, found separately
+    // per channel and for the absolute and the relative difference.  Chunk j starts at j/kShiftChunks of the image
+    // (rounded down to a multiple of lanes_used, so thread t keeps channel t % C): dark or saturated top rows do not
+    // hide the rest of the image.  Every block scans the same chunks in the same order; a channel none of them
+    // counts a sample of keeps K = 0.
     {
-        double pa[4] = {0, 0, 0, 0};
-        if (active) {
-            for (int u = 0; u < kShiftSamples; ++u) {
-                const int64_t i = (int64_t)u * lanes_used + threadIdx.x;
-                if (i >= p.n) break;
-                const Diff d = difference(p, load_raw(p, i), lo, hi, false);
-                const bool fa = !d.bad_v && fabs(d.a) < __longlong_as_double(0x7ff0000000000000LL);
-                const bool fr = !d.bad_v && fabs(d.r) < __longlong_as_double(0x7ff0000000000000LL);
-                if (fa) { pa[0] += d.a; pa[1] += 1.0; }
-                if (fr) { pa[2] += d.r; pa[3] += 1.0; }
-            }
-        }
+        const double inf = __longlong_as_double(0x7ff0000000000000LL);
         __shared__ double sh4[4][kThreads];
+        if (threadIdx.x < 4 * CL_MAX_CHANNELS) shift[threadIdx.x / CL_MAX_CHANNELS][threadIdx.x % CL_MAX_CHANNELS] = 0.0;
+        for (int chunk = 0; chunk < kShiftChunks; ++chunk) {
+            const int64_t base = chunk * (p.n / kShiftChunks) / lanes_used * lanes_used;
+            if (base >= p.n) break;
+            double pa[4] = {0, 0, 0, 0};
+            if (active) {
+                for (int u = 0; u < kShiftSamples; ++u) {
+                    const int64_t i = base + (int64_t)u * lanes_used + threadIdx.x;
+                    if (i >= p.n) break;
+                    const Diff d = difference(p, load_raw(p, i), lo, hi, USE_STD);
+                    bool fa = !d.bad_v && fabs(d.a) < inf, fr = !d.bad_v && fabs(d.r) < inf;
+                    if (USE_STD) {                       // the weight 1/sqrt(q) is finite and positive
+                        fa = fa && !d.bad_sa && d.qa > 0.0 && d.qa < inf;
+                        fr = fr && !d.bad_sr && d.qr > 0.0 && d.qr < inf;
+                    }
+                    if (fa) { pa[0] += d.a; pa[1] += 1.0; }
+                    if (fr) { pa[2] += d.r; pa[3] += 1.0; }
+                }
+            }
 #pragma unroll
-        for (int q = 0; q < 4; ++q) sh4[q][threadIdx.x] = pa[q];
-        __syncthreads();
-        if (threadIdx.x < 4 * C) {
-            const int q = threadIdx.x / C, cc = threadIdx.x % C;
-            double t = 0.0;
-            for (int l = cc; l < lanes_used; l += C) t += sh4[q][l];
-            shift[q][cc] = t;
+            for (int q = 0; q < 4; ++q) sh4[q][threadIdx.x] = pa[q];
+            __syncthreads();
+            bool pending = false;
+            if (threadIdx.x < 2 * C) {                       // (which, channel): the first chunk with a count wins
+                const int q = 2 * (threadIdx.x / C), cc = threadIdx.x % C;
+                double s = 0.0, k = 0.0;
+                for (int l = cc; l < lanes_used; l += C) { s += sh4[q][l]; k += sh4[q + 1][l]; }
+                if (shift[q + 1][cc] == 0.0) { shift[q][cc] = s; shift[q + 1][cc] = k; }
+                pending = shift[q + 1][cc] == 0.0;
+            }
+            if (!__syncthreads_or(pending)) break;
         }
         __syncthreads();
     }
@@ -324,9 +355,14 @@ __global__ void pair_final_kernel(const double* __restrict__ partial, int n_bloc
     double q = fma(dm * dm, T0, fma(-2.0 * dm, T1, T2));                      // sum w (v - mean)^2
     if (q < 0.0) q = 0.0;
     // degenerate means, as np.nansum sees them: (v - NaN)^2 is NaN for every sample -> an empty sum; (v - inf)^2 is
-    // inf for every finite v
+    // inf for every finite v and NaN for v = inf, and T0 is the weight of the samples with finite values.  Without
+    // uncertainty images np.nanstd's plain sum keeps the NaN of inf - inf or of a NaN mean: the std is NaN.  (This
+    // takes the infinity to come from an infinite sample.  A mean that overflows from finite values, |v| ~ 1e305,
+    // gives NaN here where np.nanstd gives inf; the sums cannot tell the two apart.)
+    const double inf = __longlong_as_double(0x7ff0000000000000LL);
     if (mean != mean) q = 0.0;
-    else if (fabs(mean) == __longlong_as_double(0x7ff0000000000000LL)) q = T0 > 0.0 ? fabs(mean) : 0.0;
+    else if (fabs(mean) == inf) q = T0 > 0.0 ? inf : 0.0;
+    if (!use_std && !(fabs(mean) < inf)) q = __longlong_as_double(0x7ff8000000000000LL);
     stats[(which * 3 + 0) * C + c] = mean;
     stats[(which * 3 + 1) * C + c] = sqrt(q / denom);
     stats[(which * 3 + 2) * C + c] = use_std ? totals[(which * 4 + 2) * C + c] / totals[(which * 4 + 3) * C + c]
@@ -355,6 +391,7 @@ int cl_pair_statistics(const double* x_val, const double* x_std, const double* y
     PairArgs p;
     p.x_val = x_val; p.x_std = x_std; p.y_val = y_val; p.y_std = y_std;
     p.multiplier = multiplier; p.n = n_samples; p.C = channels;
+    p.t2_multiplier = multiplier == 0.0 ? 1.0 : multiplier;
     p.has_thr = lower != nullptr;
     for (int c = 0; c < CL_MAX_CHANNELS; ++c) {      // HOST arrays of per-channel limits
         p.lower[c] = (lower && c < channels) ? lower[c] : 0.0;
