@@ -91,6 +91,9 @@ SIGNATURES = {
     "cl_welford_finalize": (_i, [_vp, _vp, _i64, _i64, _d, _vp, _vp, _vp]),
     "cl_welford_stack_workspace_bytes": (_sz, [_i, _i64]),
     "cl_welford_stack": (_i, [_vp, _i, _i64, _i, _vp, _d, _vp, _vp, _vp, _vp, _sz, _vp]),
+    "cl_welford_update_u16": (_i, [_vp, _i, _i64, _i, _vp, _i, _d, _vp, _vp, _i64, _vp]),
+    "cl_welford_finalize_u16": (_i, [_vp, _vp, _i64, _i64, _d, _vp, _vp, _vp]),
+    "cl_welford_stack_u16": (_i, [_vp, _i, _i64, _i, _vp, _i, _d, _vp, _vp, _vp, _vp, _sz, _vp]),
     "cl_icrf_tables_bytes": (_sz, [C.POINTER(IcrfProblem)]),
     "cl_icrf_curves": (_i, [C.POINTER(IcrfProblem), _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "cl_icrf_energy_workspace_bytes": (_sz, [C.POINTER(IcrfProblem), _i64]),

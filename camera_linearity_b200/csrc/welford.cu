@@ -12,27 +12,12 @@
 //    rint(mean*255) is decided in integers; only samples whose exact mean*255 is a half-integer
 //    (a rounding tie, where NumPy's answer depends on its rounding noise) are replayed with the
 //    exact sequential recurrence by a second small kernel.
-#include "common.cuh"
+#include "welford.cuh"
 
 namespace cl {
 namespace {
 
 constexpr int kThreads = 256;
-
-// ---- exact sequential recurrence ------------------------------------------------------------------
-struct WelfordState {
-    double mean, m2;
-};
-
-// video_processing.py:205-208 with n as a double and rn = RN(1/n)
-__device__ __forceinline__ void welford_step(WelfordState& s, double x, double n, double rn) {
-    const double delta = __dsub_rn(x, s.mean);
-    const double q0 = __dmul_rn(delta, rn);
-    const double rem = __fma_rn(-q0, n, delta);
-    const double q = __fma_rn(rem, rn, q0);          // == RN(delta / n)
-    s.mean = __dadd_rn(s.mean, q);
-    s.m2 = __dadd_rn(s.m2, __dmul_rn(delta, __dsub_rn(x, s.mean)));
-}
 
 // x = frame / MAX_DN (video_processing.py:203) or ICRF[frame, c] (:201)
 __global__ void __launch_bounds__(kThreads)
@@ -102,11 +87,6 @@ __global__ void welford_finalize_kernel(const double* __restrict__ mean, const d
 // Thread <-> 16 consecutive samples (one uint4 per frame).  `slices` lanes of a warp share the same
 // samples and take frames f = slice, slice + slices, ...; lanes with equal slice read consecutive
 // 16-byte vectors (coalesced).  Partial integer sums are combined with __shfl_xor.
-struct StackHeader {
-    unsigned int tie_count;
-    unsigned int pad[3];
-};
-
 __device__ __forceinline__ void accumulate_word(uint32_t x, uint32_t* s, uint32_t* q) {
     s[0] = __dp4a(x, 0x00000001u, s[0]);
     s[1] = __dp4a(x, 0x00000100u, s[1]);
@@ -263,13 +243,6 @@ constexpr int kReplayWindow = 256;
 constexpr int kReplayWarps = 4;
 constexpr int kReplayBatch = 16;
 constexpr uint32_t kLaneModeTies = 256;      // below this the warp-per-tie form has nothing to lose
-
-__device__ __forceinline__ void welford_mean_step(double& mean, double x, double n, double rn) {
-    const double delta = __dsub_rn(x, mean);          // welford_step without M2 (the replay only decides the mean)
-    const double q0 = __dmul_rn(delta, rn);
-    const double rem = __fma_rn(-q0, n, delta);
-    mean = __dadd_rn(mean, __fma_rn(rem, rn, q0));
-}
 
 __global__ void __launch_bounds__(kReplayWarps * 32)
 welford_tie_replay_kernel(const uint8_t* __restrict__ frames, int F, int64_t n, int C,
@@ -525,13 +498,6 @@ welford_stack_lut_kernel(const uint8_t* __restrict__ frames, int F, int64_t n, i
             if (mean_u8) mean_u8[base + j] = (uint8_t)wrap_bin(scaled, 0xFFu);
         }
     }
-}
-
-inline unsigned grid_for(int64_t items, int threads, int per_sm) {
-    int64_t b = (items + threads - 1) / threads;
-    const int64_t cap = (int64_t)sm_count() * per_sm;
-    if (b > cap) b = cap;
-    return (unsigned)(b < 1 ? 1 : b);
 }
 
 constexpr uint32_t kMaxFramesStack = 1000000;   // tie analysis bound, see DESIGN.md

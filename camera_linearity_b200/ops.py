@@ -345,71 +345,112 @@ def flat_field_normalize(val: Tensor, std: Tensor, flat_val: Tensor, flat_std: T
 
 
 # ------------------------------------------------------------------------------------- K3
+WELFORD_U16_MAX_FRAMES = 65536     # the stack form's limit for uint16 frames (DESIGN.md, K3); beyond: streaming form
+_U16_TABLE_ROWS = 65536
+
+
+def _welford_frames(frames: Tensor) -> Tensor:
+    if frames.dtype not in (torch.uint8, torch.uint16) or frames.ndim < 2:
+        raise TypeError("frames must be a uint8 or uint16 tensor (F, ...)")
+    return frames.contiguous()
+
+
+def _welford_table(icrf: Optional[Tensor], channels: int, wide: bool) -> Tuple[Optional[Tensor], int]:
+    """The ICRF as a contiguous float64 (rows, C) table and its row count; a uint16 stack takes up to 65536 rows."""
+    if icrf is None:
+        return None, 0
+    lut, _ = _lut_pair(icrf, None, channels)
+    rows = int(lut.shape[0])
+    if wide and not 1 <= rows <= _U16_TABLE_ROWS:
+        raise ValueError(f"an ICRF for uint16 frames has 1 ... 65536 rows, got {rows}")
+    return lut, rows
+
+
+def _dn_out_of_range() -> IndexError:
+    return IndexError("a frame's digital number has no row in the ICRF (index out of bounds, as NumPy raises)")
+
+
 @_on_device
 def welford_update(frames: Tensor, mean: Tensor, m2: Tensor, count0: int,
                    icrf: Optional[Tensor] = None, max_dn: float = 255.0) -> int:
-    """Fold ``frames`` (F, H, W, C) uint8 into the running (mean, m2) state in place -- the
-    reference's sequential recurrence (video_processing.py:205-208), bit-identical float64."""
+    """Fold ``frames`` (F, H, W, C) uint8 or uint16 into the running (mean, m2) state in place -- the
+    reference's sequential recurrence (video_processing.py:205-208), bit-identical float64.  With uint16 frames and
+    an ICRF shorter than 65536 rows, a DN without a row raises IndexError before the state changes."""
     _require_cuda(frames, mean, m2, icrf)
     lib = _lib.load()
-    if frames.dtype != torch.uint8 or frames.ndim < 2:
-        raise TypeError("frames must be a uint8 tensor (F, ...)")
-    fr = frames.contiguous()
+    fr = _welford_frames(frames)
+    wide = fr.dtype == torch.uint16
     f = int(fr.shape[0])
     n = fr[0].numel() if f else mean.numel()
     c = int(fr.shape[-1])
     for s in (mean, m2):
         if s.dtype != torch.float64 or not s.is_contiguous() or s.numel() != n:
             raise ValueError("mean / m2 must be contiguous float64 with one element per sample")
-    lut = None
-    if icrf is not None:
-        lut, _ = _lut_pair(icrf, None, c)
-    check(lib.cl_welford_update(_ptr(fr), f, n, c, _ptr(lut), float(max_dn), _ptr(mean), _ptr(m2),
-                                int(count0), _stream()), "cl_welford_update")
+    lut, rows = _welford_table(icrf, c, wide)
+    if not wide:
+        check(lib.cl_welford_update(_ptr(fr), f, n, c, _ptr(lut), float(max_dn), _ptr(mean), _ptr(m2),
+                                    int(count0), _stream()), "cl_welford_update")
+        return count0 + f
+    if lut is not None and rows < _U16_TABLE_ROWS and fr.numel() and _max_dn(fr) >= rows:
+        raise _dn_out_of_range()
+    check(lib.cl_welford_update_u16(_ptr(fr), f, n, c, _ptr(lut), rows, float(max_dn), _ptr(mean), _ptr(m2),
+                                    int(count0), _stream()), "cl_welford_update_u16")
     return count0 + f
 
 
 @_on_device
-def welford_finalize(mean: Tensor, m2: Optional[Tensor], count: int, max_dn: float = 255.0):
-    """Returns (sem float64 or None, mean_u8) -- video_processing.py:210-215 with repair R9."""
+def welford_finalize(mean: Tensor, m2: Optional[Tensor], count: int, max_dn: float = 255.0,
+                     dtype: torch.dtype = torch.uint8):
+    """Returns (sem float64 or None, quantised mean) -- video_processing.py:210-215 with repair R9.  The quantised
+    mean is ``np.around(mean * max_dn).astype(dtype)``: ``dtype`` torch.uint8 (8-bit frames) or torch.uint16 (16-bit
+    frames, the R9 extension of DESIGN.md section 3)."""
     _require_cuda(mean, m2)
+    if dtype not in (torch.uint8, torch.uint16):
+        raise TypeError(f"the quantised mean is uint8 or uint16, not {dtype}")
     lib = _lib.load()
     n = mean.numel()
     sem = torch.empty_like(mean) if m2 is not None else None
-    mean_u8 = torch.empty(mean.shape, dtype=torch.uint8, device=mean.device)
-    check(lib.cl_welford_finalize(_ptr(mean), _ptr(m2), int(count), n, float(max_dn), _ptr(sem),
-                                  _ptr(mean_u8), _stream()), "cl_welford_finalize")
-    return sem, mean_u8
+    mean_q = torch.empty(mean.shape, dtype=dtype, device=mean.device)
+    fn = lib.cl_welford_finalize_u16 if dtype == torch.uint16 else lib.cl_welford_finalize
+    check(fn(_ptr(mean), _ptr(m2), int(count), n, float(max_dn), _ptr(sem), _ptr(mean_q), _stream()),
+          "cl_welford_finalize_u16" if dtype == torch.uint16 else "cl_welford_finalize")
+    return sem, mean_q
 
 
 @_on_device
 def welford_stack(frames: Tensor, icrf: Optional[Tensor] = None, max_dn: float = 255.0,
                   workspace: Optional[Tensor] = None):
-    """Mean / SEM / uint8 mean of a resident frame stack (F, H, W, C) uint8 (K3 of DESIGN.md)."""
+    """Mean / SEM / quantised mean of a resident frame stack (F, H, W, C) uint8 or uint16 (K3 of DESIGN.md).  The
+    quantised mean has the frames' dtype.  uint16 stacks of more than WELFORD_U16_MAX_FRAMES frames raise
+    CamlinError (CL_ERR_UNSUPPORTED): ``video_processing.welford_stack`` takes the streaming form for them."""
     _require_cuda(frames, icrf)
     lib = _lib.load()
-    if frames.dtype != torch.uint8 or frames.ndim < 2:
-        raise TypeError("frames must be a uint8 tensor (F, ...)")
-    fr = frames.contiguous()
+    fr = _welford_frames(frames)
+    wide = fr.dtype == torch.uint16
     f = int(fr.shape[0])
     if f < 1:
         raise ValueError("at least one frame is required")
     shape = tuple(fr.shape[1:])
     n = fr[0].numel()
     c = int(fr.shape[-1])
-    lut = None
-    if icrf is not None:
-        lut, _ = _lut_pair(icrf, None, c)
+    lut, rows = _welford_table(icrf, c, wide)
     mean = torch.empty(shape, dtype=torch.float64, device=fr.device)
     sem = torch.empty_like(mean)
-    mean_u8 = torch.empty(shape, dtype=torch.uint8, device=fr.device)
+    mean_q = torch.empty(shape, dtype=fr.dtype, device=fr.device)
     ws_bytes = lib.cl_welford_stack_workspace_bytes(f, n)
     ws = workspace
     if ws is None or ws.numel() * ws.element_size() < ws_bytes:
         ws = torch.empty(ws_bytes, dtype=torch.uint8, device=fr.device)
-    check(lib.cl_welford_stack(_ptr(fr), f, n, c, _ptr(lut), float(max_dn), _ptr(mean), _ptr(sem),
-                               _ptr(mean_u8), _ptr(ws), ws_bytes, _stream()), "cl_welford_stack")
-    return mean, sem, mean_u8
+    if not wide:
+        check(lib.cl_welford_stack(_ptr(fr), f, n, c, _ptr(lut), float(max_dn), _ptr(mean), _ptr(sem),
+                                   _ptr(mean_q), _ptr(ws), ws_bytes, _stream()), "cl_welford_stack")
+        return mean, sem, mean_q
+    check(lib.cl_welford_stack_u16(_ptr(fr), f, n, c, _ptr(lut), rows, float(max_dn), _ptr(mean), _ptr(sem),
+                                   _ptr(mean_q), _ptr(ws), ws_bytes, _stream()), "cl_welford_stack_u16")
+    # a table shorter than 65536 rows: the kernel flags DNs without a row in the workspace header's second word
+    if lut is not None and rows < _U16_TABLE_ROWS and n and bool(ws.reshape(-1).view(torch.uint8)[4:8].any()):
+        raise _dn_out_of_range()
+    return mean, sem, mean_q
 
 
 # ------------------------------------------------------------------------------------- K4
@@ -896,6 +937,13 @@ def _op_welford_update(frames: Tensor, mean: Tensor, m2: Tensor, count0: int, ic
 def _op_welford_finalize(mean: Tensor, m2: Tensor, count: int, max_dn: float) -> List[Tensor]:
     sem, mean_u8 = welford_finalize(mean, m2, count, max_dn)
     return [sem, mean_u8]
+
+
+@torch.library.custom_op("camera_linearity::welford_finalize_u16", mutates_args=(), device_types="cuda")
+def _op_welford_finalize_u16(mean: Tensor, m2: Tensor, count: int, max_dn: float) -> List[Tensor]:
+    """welford_finalize with the uint16 mean of 16-bit frames."""
+    sem, mean_u16 = welford_finalize(mean, m2, count, max_dn, torch.uint16)
+    return [sem, mean_u16]
 
 
 @torch.library.custom_op("camera_linearity::gaussian_weight", mutates_args=(), device_types="cuda")

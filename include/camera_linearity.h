@@ -173,6 +173,24 @@ int cl_welford_stack(const uint8_t* frames, int n_frames, int64_t n_samples, int
                      const double* lut, double max_dn, double* mean, double* sem,
                      uint8_t* mean_u8, void* workspace, size_t workspace_bytes, void* stream);
 
+/* K3 for 16-bit cameras (16-bit data, or 12-bit data stored in uint16): the same three calls for
+ * [F][n_samples] uint16 frames.  lut (nullable) is [lut_rows][C] float64 with 1 <= lut_rows <= 65536
+ * (ignored without a table); a DN >= lut_rows reads the last row, and cl_welford_stack_u16 then sets the
+ * second uint32 of the workspace to nonzero (the caller reports it; it cannot happen with 65536 rows).
+ * The quantised mean is uint16: np.around(mean * max_dn).astype(np.uint16), wrapping cast, NaN -> 0.
+ * cl_welford_stack_u16 takes up to 65536 frames (its tie analysis, see DESIGN.md) and returns
+ * CL_ERR_UNSUPPORTED beyond, where the streaming form applies; its workspace is
+ * cl_welford_stack_workspace_bytes.  frames must be 2-byte aligned, float buffers 8-byte aligned
+ * (CL_ERR_ALIGNMENT otherwise); other alignments and ragged n take an exact replay of every sample. */
+int cl_welford_update_u16(const uint16_t* frames, int n_frames, int64_t n_samples, int channels,
+                          const double* lut, int lut_rows, double max_dn, double* mean, double* m2,
+                          int64_t count0, void* stream);
+int cl_welford_finalize_u16(const double* mean, const double* m2, int64_t count, int64_t n_samples,
+                            double max_dn, double* sem, uint16_t* mean_u16, void* stream);
+int cl_welford_stack_u16(const uint16_t* frames, int n_frames, int64_t n_samples, int channels,
+                         const double* lut, int lut_rows, double max_dn, double* mean, double* sem,
+                         uint16_t* mean_u16, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---------------------------------------------------------------------------------------------
  * K4  ICRF calibration objective for a whole differential-evolution population -- replaces
  *     _inverse_camera_response_function (modules/ICRF_calibration_exposure.py:20-44),
