@@ -48,13 +48,23 @@ constexpr int kMaxN = CL_MAX_PAIR_EXPOSURES;
 
 __host__ __device__ inline int n_pairs(int n) { return n * (n - 1) / 2; }
 
-// see the file header: lower >= 1 makes the range masks a property of the DN alone
-__host__ __device__ inline bool uniform_masks(const cl_icrf_problem& p) { return p.lower >= 1; }
+// see the file header: lower >= 1 makes the range masks a property of the DN alone.  Swapped limits (upper < lower)
+// mask every sample of a candidate that passes the gates; the NaN-checking path gives that +inf, while the uniform
+// pixel loop's unsigned span test would wrap and count the DNs outside (upper, lower) as valid.
+__host__ __device__ inline bool uniform_masks(const cl_icrf_problem& p) { return p.lower >= 1 && p.lower <= p.upper; }
 
 struct ExposureScales {
     double inv_t[kMaxN];              // 1 / t_k
     double t[kMaxN];
 };
+
+// R-table entry of an unmasked point on the uniform path.  A subnormal curve value has 1/v = inf, and the weighted
+// loop's fma(|u - 1|, w = 0, num) would turn the whole pair sum into NaN; the reference gives such a pair the weight
+// 0 (its propagated sigma overflows), which R = 0 reproduces exactly: u = t1 = t2 = 0, so var = 0 and w = 0.
+__device__ __forceinline__ double reciprocal(const cl_icrf_problem& prob, double v) {
+    const double r = 1.0 / v;
+    return prob.use_std && isinf(r) ? 0.0 : r;
+}
 
 // ---- candidate curves, gates and tables -----------------------------------------------------------
 // One CTA per candidate, one thread per curve point.  `p` points at the candidate's parameters (global or
@@ -108,7 +118,7 @@ __device__ __forceinline__ void build_curve(const cl_icrf_problem& prob, const d
             // zero-variance pairs and walk its pixels a second time.  It gets the benign table 1 on [lower, upper].
             const bool inside = d >= prob.lower && d <= prob.upper;
             tables[at] = bad ? (inside ? 1.0 : 0.0) : (masked ? 0.0 : v);
-            tables[(int64_t)prob.n_candidates * D + at] = bad ? (inside ? 1.0 : 0.0) : (masked ? 0.0 : 1.0 / v);
+            tables[(int64_t)prob.n_candidates * D + at] = bad ? (inside ? 1.0 : 0.0) : (masked ? 0.0 : reciprocal(prob, v));
         } else {
             const double m = masked ? __longlong_as_double(0x7ff8000000000000LL) : v;
             tables[at] = m;
@@ -196,7 +206,7 @@ __device__ __forceinline__ void store_point(const cl_icrf_problem& prob, int s, 
         // zero-variance pairs and walk its pixels a second time.  It gets the benign table 1 on [lower, upper].
         const bool inside = d >= prob.lower && d <= prob.upper;
         tables[at] = bad ? (inside ? 1.0 : 0.0) : (masked ? 0.0 : v);
-        tables[(int64_t)prob.n_candidates * D + at] = bad ? (inside ? 1.0 : 0.0) : (masked ? 0.0 : 1.0 / v);
+        tables[(int64_t)prob.n_candidates * D + at] = bad ? (inside ? 1.0 : 0.0) : (masked ? 0.0 : reciprocal(prob, v));
     } else {
         const double m = masked ? __longlong_as_double(0x7ff8000000000000LL) : v;
         tables[at] = m;

@@ -991,6 +991,8 @@ def _op_icrf_energy_partial(tables: Tensor, dn: Tensor, std: Optional[Tensor], e
     if dn.dtype not in (torch.uint8, torch.uint16) or dn.ndim != 2:
         raise TypeError("dn must be a (pixels, N) uint8 or uint16 tensor")
     n_px, n_exp = (int(v) for v in dn.shape)
+    if n_px and _max_dn(dn) >= datapoints:          # the kernel would read the curve's last row instead
+        raise IndexError("digital numbers exceed the curve length")
     prob = _icrf_problem(n_candidates, n_params, datapoints, use_mean, lower, upper, n_exp, std is not None)
     sd = None if std is None else _f64c(std)
     acc = torch.empty((n_candidates, n_exp * (n_exp - 1) // 2, 2), dtype=torch.float64, device=dn.device)

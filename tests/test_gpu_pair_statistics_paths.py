@@ -542,10 +542,15 @@ def test_dispatch_map():
     with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
         torch.ones(1, device="cuda").add_(1)
         torch.cuda.synchronize()
-        for _, (hx, hy, m), _ in DISPATCH:
-            _run(x, s if hx else None, y, s if hy else None, m)
+        for _ in range(2):                    # with many modules loaded, tracing can start late in the session
+            for _, (hx, hy, m), _ in DISPATCH:
+                _run(x, s if hx else None, y, s if hy else None, m)
+            torch.cuda.synchronize()
     events = sorted(prof.events(), key=lambda e: e.time_range.start)
     got = [n for n in (_kernel_name(e.name) for e in events) if n]
     if not events:
         pytest.skip("the profiler records no device activity here")
-    assert got == [k for _, _, kernel in DISPATCH for k in (kernel, "pair_final_kernel")]
+    want = [k for _, _, kernel in DISPATCH for k in (kernel, "pair_final_kernel")]
+    assert got[-len(want):] == want                                       # the second pass, exactly
+    first = got[: len(got) - len(want)]
+    assert len(first) <= len(want) and first == want[len(want) - len(first):]
