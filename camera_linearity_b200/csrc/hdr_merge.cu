@@ -327,7 +327,7 @@ dark_scan_kernel(const __grid_constant__ MergeParams p) {
 }
 
 // The single-pass kernel's rule for one sample (hdr_merge_stream.cu): the expanded variance, unless it cancelled
-// (q < kStreamCancel * A), in which case the exact two-pass formula.  Same operations in the same order as the
+// (expansion_cancelled), in which case the exact two-pass formula.  Same operations in the same order as the
 // kernel, so a sample gets the same bits whichever of the two computes it.
 __device__ __noinline__ void recompute_sample_stream(const MergeParams& p, int64_t i) {
     const int C = p.C;
@@ -356,7 +356,7 @@ __device__ __noinline__ void recompute_sample_stream(const MergeParams& p, int64
     }
     const double rS = 1.0 / S;
     const double q = expanded_variance(A, B, Cc, rS);
-    if (q < kStreamCancel * A) {
+    if (expansion_cancelled(q, A, B, Cc, rS)) {
         recompute_sample<uint8_t>(p, i);
         return;
     }

@@ -48,9 +48,8 @@ struct MergeParams {
                                // (hdr_merge_stream.cu), 2 = STD table (hdr_merge_stream_lut.cu)
 };
 
-// single-pass kernel: a sample whose expanded variance q kept less than this fraction of its largest term A has
-// cancelled by more than 6 digits and is recomputed with the exact two-pass formula; above it the expansion is within
-// 1.1e-16 / kStreamCancel = 1.1e-10 of the two-pass result
+// single-pass kernel: a sample whose expanded variance q kept less than this fraction of the scale of its rounding error,
+// A + 2|B| rS + C rS^2 (expansion_cancelled), is recomputed with the exact two-pass formula
 constexpr double kStreamCancel = 1e-6;
 
 constexpr size_t kHotListHeader = 4;   // uint32 entries reserved in front of the list (counter + pad)
@@ -136,6 +135,15 @@ __device__ __forceinline__ void merge_accumulate_expanded_lut(double w, double p
 __device__ __forceinline__ double expanded_variance(double A, double B, double C, double rS) {
     const double q = fma(rS * rS, C, fma(-2.0 * rS, B, A));
     return q < 0.0 ? 0.0 : q;           // (NaN compares false and is kept)
+}
+
+// The fix-up rule of the single-pass kernels (and of recompute_sample_stream, which must agree bit for bit).  The
+// rounding error of q = A - 2B rS + C rS^2 is about u L (A + 2|B| rS + C rS^2), L the longest chain of additions, so
+// a sample is flagged when q kept less than kStreamCancel of that scale: an unflagged uncertainty is then within
+// u L / (2 kStreamCancel) of the exact one in the worst case and within 1e-9 as measured (DESIGN.md, K2).  A test against
+// A alone let samples with C rS^2 ~ B rS ~ A through at up to 4x that error.  (NaN compares false: not flagged here.)
+__device__ __forceinline__ bool expansion_cancelled(double q, double A, double B, double C, double rS) {
+    return q < kStreamCancel * fma(rS * rS, C, fma(2.0 * rS, fabs(B), A));
 }
 
 __device__ __forceinline__ double kappa_of(uint32_t d, double kappa_scale) {

@@ -13,9 +13,9 @@
 // against the 1e-6 the north star allows.  That bound covers the STRUCTURAL cancellation only: where the two parts of
 // x - e/S = dw g (1 - w/S) + w dg also cancel each other by accident, the uncertainty itself is anomalously small and
 // the expansion's absolute error (~1e-16 A) is large relative to it (1e-3 seen on 0.3 % of the samples of an
-// adversarial stack).  The kernel therefore checks q < 1e-6 A per sample and hands those samples to the exact
-// two-pass formula through the fix-up work list (merge_fixup_kernel; none on ordinary stacks): every sample is
-// within 1.1e-10 of the two-pass kernels (tests assert 1e-9), and the rule is deterministic -- the fix-up pass
+// adversarial stack).  The kernel therefore checks q < 1e-6 (A + 2|B|/S + C/S^2) per sample (expansion_cancelled) and
+// hands those samples to the exact two-pass formula through the fix-up work list (merge_fixup_kernel; none on ordinary
+// stacks): every other sample is within 1e-9 of the exact result (tests), and the rule is deterministic -- the fix-up pass
 // applies the same expansion + check, so a sample gets the same bits whichever kernel computes it.  N = 1 has no
 // weight floor and stays on the two-pass kernels.
 //
@@ -271,8 +271,8 @@ merge_stream_kernel(const __grid_constant__ MergeParams p, const StreamLayout L,
             double v0 = av0 * r0, v1 = av1 * r1, v2 = av2 * r2;
             const double q0 = expanded_variance(A0, B0, C0, r0), q1 = expanded_variance(A1, B1, C1, r1),
                          q2 = expanded_variance(A2, B2, C2, r2);
-            bool f0 = q0 < kStreamCancel * A0 || !k0, f1 = q1 < kStreamCancel * A1 || !k1,
-                 f2 = q2 < kStreamCancel * A2 || !k2;
+            bool f0 = expansion_cancelled(q0, A0, B0, C0, r0) || !k0, f1 = expansion_cancelled(q1, A1, B1, C1, r1) || !k1,
+                 f2 = expansion_cancelled(q2, A2, B2, C2, r2) || !k2;
             double u0, u1, u2;
             if (has_flat) {
                 mbar_wait(&c_full[s], phase);

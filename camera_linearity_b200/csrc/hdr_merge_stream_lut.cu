@@ -256,8 +256,8 @@ merge_stream_lut_kernel(const __grid_constant__ MergeParams p, const SLutLayout 
             double v0 = av0 * r0, v1 = av1 * r1, v2 = av2 * r2;
             const double q0 = expanded_variance(A0, B0, C0, r0), q1 = expanded_variance(A1, B1, C1, r1),
                          q2 = expanded_variance(A2, B2, C2, r2);
-            bool c0 = q0 < kStreamCancel * A0 || !k0, c1f = q1 < kStreamCancel * A1 || !k1,
-                 c2f = q2 < kStreamCancel * A2 || !k2;
+            bool c0 = expansion_cancelled(q0, A0, B0, C0, r0) || !k0, c1f = expansion_cancelled(q1, A1, B1, C1, r1) || !k1,
+                 c2f = expansion_cancelled(q2, A2, B2, C2, r2) || !k2;
             double u0, u1, u2;
             if (has_flat) {
                 double rf0, rf1, rf2;
